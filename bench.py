@@ -1,12 +1,17 @@
 #!/usr/bin/env python
 """bench.py -- the driver's measurement contract for the pairwise-contraction hot path.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json: "pairwise contractions/sec + effective ZGEMM TFLOP/s on random-circuit network"; north star:
 the 36-qubit random-circuit amplitude network): `random_circuit(36 qubits, 10 rounds, p1 = p2 = 0.5, Sycamore coupling,
 seed 1)` closed with <0| bras -> 489 leaves, 488 pairwise contractions.  A "step" is ONE full contraction of that network
-through `contract_tensor_network`.
+through `contract_tensor_network`; K steps are timed in each of the two forms below (value and e2e).
+
+--dump-outputs DIR writes, after the timed steps, what the last step of each form returned on rank 0: DIR/amplitude.npy
+(value) and DIR/amplitude_e2e.npy (e2e), each the complex amplitude as float64 [re, im]; --impl reference writes its
+own DIR/amplitude.npy.  The network and path are fixed by the seed, so two builds run with the same arguments can be
+compared output for output.
 
   N = 1   greedy (Cotengrust) path, 6.7e12 flop.
           value = pairs/s with the leaves resident in HBM (tncb_plan_stage + tncb_plan_run),
@@ -238,6 +243,14 @@ def _captured_traffic():
     return None, None
 
 
+def dump_outputs(directory, outputs):
+    """Each complex output as DIR/<name>.npy, float64 with a trailing [re, im] axis."""
+    os.makedirs(directory, exist_ok=True)
+    for name, z in outputs.items():
+        z = np.asarray(z, dtype=np.complex128)
+        np.save(os.path.join(directory, name + ".npy"), np.stack([z.real, z.imag], axis=-1))
+
+
 def oracle_network_seconds(tn, path, repeats, warm=1):
     import torch
     from oracle import tnc_oracle as orc
@@ -270,6 +283,8 @@ def run_reference(args):
         mode = f"partitioned into {world} parts (tools/plan_partitions.py), local paths then the fan-in pairs, sequentially on the host"
     pairs, flops = count_pairs(path), path_flops(net, path)
     ts, amp = oracle_network_seconds(net, path, args.steps, warm=max(1, args.warmup))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"amplitude": amp})
     sec = float(np.mean(ts))
     val = pairs / sec
     line = {
@@ -467,7 +482,7 @@ def run_ours(args):
     value = pairs / (ms_per_step * 1e-3)
 
     # ---- e2e: the public call from host leaves, device->host read of the amplitude inside -----------------
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
     for _ in range(warmup):       # W >= 3 like the resident form: the library compiles its plan on the SECOND sighting of a structure
         read_amp(step_e2e())
     barrier()
@@ -482,6 +497,8 @@ def run_ours(args):
     e2e_ms = max_over_ranks(ev0.elapsed_time(ev1)) / e2e_steps
     e2e_wall_ms = max_over_ranks((w1 - w0) * 1e3) / e2e_steps
     e2e_val = pairs / (e2e_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"amplitude": amp, "amplitude_e2e": amp_e2e})
 
     line = None
     if rank == 0:
@@ -686,14 +703,21 @@ def parity_and_modes(tb, ctx, dist, torch, stream, tn, fpath, net, path, amp_fan
 
 def main():
     ap = argparse.ArgumentParser()
+    def positive(s):
+        n = int(s)
+        if n < 1:
+            raise argparse.ArgumentTypeError(f"must be >= 1, got {n}")
+        return n
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=positive, default=20, help="timed full contractions of the headline network, in each form")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-pair", action="store_true", help="skip the pair_c2 object")
     ap.add_argument("--no-extras", action="store_true", help="skip the extra objects")
     ap.add_argument("--no-config5", action="store_true", help="skip the Sycamore-53 depth-12 object (about 30 s at N = 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float64 [re, im])")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -1,21 +1,21 @@
 """Generates tests/golden/contraction_kat.json from the reference's own golden vectors.
 
-Run in the build container (the GPU box has no /root/reference):
-    python tests/golden/make_golden.py
-Source: /root/reference/tnc/src/tensornetwork/contraction_test_data.json, the data file of
+    python tests/golden/make_golden.py <path to a qc-tum/TNC checkout>
+
+Source: tnc/src/tensornetwork/contraction_test_data.json in that checkout, the data file of
 test_tensor_contraction / test_tn_contraction (tnc/src/tensornetwork/contraction.rs:121-224).
 The values are copied verbatim (repr round-trips float64 exactly); only the JSON layout is
-compacted (re/im pairs -> two flat lists per tensor).
+compacted (re/im pairs -> two flat lists per tensor).  The tests read only the generated file.
 """
 import json
 import os
+import sys
 
-SRC = "/root/reference/tnc/src/tensornetwork/contraction_test_data.json"
 DST = os.path.join(os.path.dirname(os.path.abspath(__file__)), "contraction_kat.json")
 
 
-def main():
-    with open(SRC) as f:
+def main(tnc_checkout):
+    with open(os.path.join(tnc_checkout, "tnc", "src", "tensornetwork", "contraction_test_data.json")) as f:
         data = json.load(f)
     out = {"_source": "tnc/src/tensornetwork/contraction_test_data.json @ qc-tum/TNC 5dd62b3",
            "_epsilon": 1e-14, "tensors": {}}
@@ -30,4 +30,6 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    main(sys.argv[1])

@@ -1,7 +1,8 @@
 """HDF5 tensor files (tnc/src/io/hdf5.rs) through the C ABI (tncb_hdf5_*, csrc/hdf5io.cpp) -- host only, no GPU.
 
 Pinning, since neither libhdf5 nor a byte-level fixture of the reference exists here:
-  * a file written by libhdf5 itself that ships with this image (scipy's MATLAB-7.3 test fixture) is read correctly;
+  * a file written by libhdf5 itself (tests/golden/testhdf5_7.4_GLNX86.mat, SciPy 1.18.1's BSD-licensed MATLAB-7.3 test
+    fixture scipy/io/matlab/tests/data/testhdf5_7.4_GLNX86.mat, stored verbatim) is read correctly;
   * the writer's output is walked by an independent pure-Python restatement of the format (tests/h5check.py::parse_v0),
     which asserts what libhdf5 relies on when it opens such a file;
   * files emitted by a second independent builder in the encodings of newer libhdf5 objects (h5check.LatestFile) are read
@@ -19,14 +20,7 @@ import pytest
 import h5check
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SCIPY_FIXTURE = None
-try:
-    import scipy.io
-    _p = os.path.join(os.path.dirname(scipy.io.__file__), "matlab", "tests", "data", "testhdf5_7.4_GLNX86.mat")
-    if os.path.exists(_p):
-        SCIPY_FIXTURE = _p
-except Exception:  # pragma: no cover
-    pass
+LIBHDF5_FIXTURE = os.path.join(ROOT, "tests", "golden", "testhdf5_7.4_GLNX86.mat")
 
 
 @pytest.fixture(scope="module")
@@ -40,11 +34,10 @@ def cplx(rng, shape):
 
 
 # ---------------------------------------------------------------- a file libhdf5 wrote
-@pytest.mark.skipif(SCIPY_FIXTURE is None, reason="scipy's HDF5 fixture is not installed")
 def test_reads_a_file_written_by_libhdf5(h5):
     """512-byte user block, superblock 0 with a base address, symbol-table root group, version-1 object header with a
     version-1 fill value, version-2 data layout, IEEE f64 dataset 0:pi/4:2pi of shape (9, 1)."""
-    with h5.Hdf5File(SCIPY_FIXTURE, "/") as f:
+    with h5.Hdf5File(LIBHDF5_FIXTURE, "/") as f:
         assert f.member_names() == ["testdouble"]
         assert f.shape(0) == [9, 1]
         got = f.read(0)
@@ -54,7 +47,7 @@ def test_reads_a_file_written_by_libhdf5(h5):
     # the same file has no /tensors group
     from tnc_b200 import TncbError
     with pytest.raises(TncbError) as e:
-        h5.load_data(SCIPY_FIXTURE)
+        h5.load_data(LIBHDF5_FIXTURE)
     assert e.value.status == -10 and "tensors" in str(e.value)
 
 

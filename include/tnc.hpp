@@ -92,12 +92,19 @@ struct Tensor {
   void push_tensor(Tensor t) { tensors.push_back(std::move(t)); }
   const Tensor& tensor(size_t i) const { return tensors.at(i); }
 
-  // `elements()`: row-major data of a contracted leaf (downloads from the device)
+  // `elements()`: row-major data of a contracted leaf (downloads from the device; complex64 results are widened)
   std::vector<Complex64> elements() const {
     if (tensordata.kind == TensorData::Matrix) return tensordata.matrix;
     if (tensordata.kind != TensorData::Device) throw Error(TNCB_ERR_UNCONTRACTED, "Cannot convert uncontracted tensor to data");
-    std::vector<Complex64> out(tncb_tensor_elements(tensordata.device->t));
-    check(tncb_tensor_download(tensordata.device->ctx, tensordata.device->t, reinterpret_cast<double*>(out.data())));
+    const tncb_tensor* t = tensordata.device->t;
+    std::vector<Complex64> out(tncb_tensor_elements(t));
+    if (tncb_tensor_dtype(t) == TNCB_C64) {
+      std::vector<std::complex<float>> narrow(out.size());
+      check(tncb_tensor_download(tensordata.device->ctx, t, reinterpret_cast<double*>(narrow.data())));
+      for (size_t i = 0; i < out.size(); i++) out[i] = Complex64(narrow[i].real(), narrow[i].imag());
+      return out;
+    }
+    check(tncb_tensor_download(tensordata.device->ctx, t, reinterpret_cast<double*>(out.data())));
     return out;
   }
 };
@@ -162,13 +169,14 @@ inline void release_device_inputs(Tensor& t) {  // the call consumed them (mem::
 }
 }  // namespace detail
 
-// Fully contracts `tn` (moved in, as in the reference) with the replace-left `path`.
-inline Tensor contract_tensor_network(Context& ctx, Tensor tn, const ContractionPath& path) {
+// Fully contracts `tn` (moved in, as in the reference) with the replace-left `path`.  dtype = TNCB_C64 runs every kernel
+// in complex64 (f64 accumulation, one rounding per result); host payloads stay complex128 and are narrowed on upload.
+inline Tensor contract_tensor_network(Context& ctx, Tensor tn, const ContractionPath& path, tncb_dtype dtype = TNCB_C128) {
   detail::Marshal m;
   tncb_tn c_tn = m.tn(tn);
   tncb_path c_path = m.path(path);
   tncb_tensor* out = nullptr; int n_out = 0; uint64_t legs[64];
-  check(tncb_contract_tensor_network(ctx.get(), &c_tn, &c_path, &out, &n_out, legs));
+  check(tncb_contract_tensor_network_dt(ctx.get(), &c_tn, &c_path, dtype, &out, &n_out, legs));
   detail::release_device_inputs(tn);
   Tensor res;
   if (!out) return res;
@@ -185,11 +193,11 @@ inline Tensor contract_tensor_network(Context& ctx, Tensor tn, const Contraction
 // schedule, the static memory layout, the batched tiny pairs and (for launch-bound networks) the CUDA graph.
 class NetworkPlan {
  public:
-  NetworkPlan(Context& ctx, const Tensor& tn, const ContractionPath& path) : ctx_(ctx) {
+  NetworkPlan(Context& ctx, const Tensor& tn, const ContractionPath& path, tncb_dtype dtype = TNCB_C128) : ctx_(ctx) {
     detail::Marshal m;
     tncb_tn c_tn = m.tn(tn);
     tncb_path c_path = m.path(path);
-    check(tncb_plan_create(ctx.get(), &c_tn, &c_path, &h_));
+    check(tncb_plan_create_dt(ctx.get(), &c_tn, &c_path, dtype, &h_));
   }
   ~NetworkPlan() { tncb_plan_destroy(h_); }
   NetworkPlan(const NetworkPlan&) = delete;

@@ -49,8 +49,20 @@ typedef enum tncb_status {
   TNCB_ERR_IO = -10           /* file missing / unreadable / not (well-formed) HDF5    */
 } tncb_status;
 
+/* Element type of a tensor, a network run or a plan.  complex128 is the default of every entry point without a
+ * dtype argument.  complex64 is always explicit (the *_dt entry points) and follows one precision contract:
+ * operands are read as complex64 and widened exactly to f64, products and sums run in f64 (in the order of the
+ * complex128 kernel), the result is rounded to complex64 once, at the store.  K0, K0-batch, K1 (DMMA) and K2 make
+ * the same kernel and configuration choices for both types, so their complex64 result equals, bit for bit,
+ * complex64(complex128 kernel(widen(a), widen(b))).  K1' (CRT) keeps a = 28 operand bits for complex64 pairs unless
+ * a tolerance is set: the bound below becomes 2^-24 K max|b[n,:]| max|a[m,:]|, the classical worst case of an FP32 dot
+ * product, with about 9 moduli at K = 4096.  complex64 pairs that qualify for K1' always use the CRT engine, also
+ * when tncb_ctx_set_tcgen05_engine(1) selected digit slicing (which has no complex64 path).
+ * Operands of different dtypes are refused with TNCB_ERR_INVALID (no implicit promotion). */
+typedef enum tncb_dtype { TNCB_C128 = 0, TNCB_C64 = 1 } tncb_dtype;
+
 typedef struct tncb_ctx tncb_ctx;       /* one device + stream + arena              */
-typedef struct tncb_tensor tncb_tensor; /* a device-resident complex128 tensor      */
+typedef struct tncb_tensor tncb_tensor; /* a device-resident complex128 or complex64 tensor */
 typedef struct tncb_plan tncb_plan;     /* a compiled (network, path) schedule      */
 typedef struct tncb_h5file tncb_h5file; /* an opened HDF5 tensor file (host only)   */
 
@@ -139,6 +151,13 @@ int tncb_ctx_gemm_totals(tncb_ctx* ctx, double* ms, double* int8_ops, uint64_t* 
 int tncb_tensor_upload(tncb_ctx* ctx, int rank, const uint64_t* dims,
                        const double* host_re_im, tncb_tensor** out);
 int tncb_tensor_alloc(tncb_ctx* ctx, int rank, const uint64_t* dims, tncb_tensor** out);
+/* Same with an element type: host_re_im holds interleaved float pairs for TNCB_C64, double pairs for TNCB_C128. */
+int tncb_tensor_upload_dt(tncb_ctx* ctx, int rank, const uint64_t* dims, int dtype, const void* host_re_im, tncb_tensor** out);
+int tncb_tensor_alloc_dt(tncb_ctx* ctx, int rank, const uint64_t* dims, int dtype, tncb_tensor** out);
+/* tncb_dtype of t (TNCB_ERR_INVALID for NULL). */
+int tncb_tensor_dtype(const tncb_tensor* t);
+/* download / write / read copy raw data in the tensor's own dtype: for a complex64 tensor the host buffer holds
+ * interleaved float pairs (8 bytes per element) although the pointer is declared double*. */
 int tncb_tensor_download(tncb_ctx* ctx, const tncb_tensor* t, double* host_re_im);
 /* Asynchronous variants on the ctx stream (host buffer should be pinned; the caller
  * synchronises with tncb_ctx_synchronize before touching it). */
@@ -148,14 +167,17 @@ int tncb_tensor_free(tncb_ctx* ctx, tncb_tensor* t);
 int tncb_tensor_rank(const tncb_tensor* t);
 int tncb_tensor_dims(const tncb_tensor* t, uint64_t* dims_out);
 uint64_t tncb_tensor_elements(const tncb_tensor* t);
-void* tncb_tensor_device_ptr(const tncb_tensor* t); /* double2*, row-major */
+void* tncb_tensor_device_ptr(const tncb_tensor* t); /* double2* (complex128) or float2* (complex64), row-major */
 
 /* ---- one pairwise contraction: replaces
  *      tetra::contract(out_legs, a_legs, a, b_legs, b) as called at
  *      tnc/src/tensornetwork/contraction.rs:78-84.  Consumes a and b (the Rust
  *      call moves them), returns a new tensor whose legs are out_legs, which must
  *      equal (b \ a) ++ (a \ b).  Pass out_legs = NULL to skip that check and
- *      read the legs back with tncb_pair_out_legs. ---- */
+ *      read the legs back with tncb_pair_out_legs.
+ *      The pair entry points, tncb_permute, tncb_conjugate and tncb_tensor_add follow their operands' dtype (the
+ *      result has it too); operands (and the output of _into) of different dtypes -> TNCB_ERR_INVALID.
+ *      tncb_contract_pair_host is complex128 only. ---- */
 int tncb_contract_pair(tncb_ctx* ctx, int n_out, const uint64_t* out_legs,
                        int n_a, const uint64_t* a_legs, tncb_tensor* a,
                        int n_b, const uint64_t* b_legs, tncb_tensor* b,
@@ -255,6 +277,12 @@ typedef struct tncb_path {
  * least recently used evicted; TNCB_PLAN_CACHE=0 disables): no schedule construction, tiny pairs batched per level. */
 int tncb_contract_tensor_network(tncb_ctx* ctx, const tncb_tn* tn, const tncb_path* path,
                                  tncb_tensor** out, int* n_out, uint64_t* out_legs);
+/* The same in a chosen element type (tncb_contract_tensor_network == dtype TNCB_C128).  tncb_tn is unchanged: host
+ * payloads (Matrix, Gate, File) stay complex128 and are narrowed to complex64 while they are written into the pinned
+ * staging block (one H2D copy of half the size).  TNCB_DATA_DEVICE leaves must already have `dtype`
+ * (TNCB_ERR_INVALID otherwise).  The plan cache keys on the dtype as well. */
+int tncb_contract_tensor_network_dt(tncb_ctx* ctx, const tncb_tn* tn, const tncb_path* path, int dtype,
+                                    tncb_tensor** out, int* n_out, uint64_t* out_legs);
 
 /* Legs and bond dimensions of the result of tncb_contract_tensor_network(tn, path), from metadata alone (host only, no
  * GPU work; the same validation and the same errors as the real call).  The fan-in needs it: only the raw buffer of a
@@ -267,6 +295,9 @@ int tncb_network_out_legs(const tncb_tn* tn, const tncb_path* path, int* n_out, 
  * (e.g. other bitstrings or angles) re-uses the schedule, arena layout and the
  * captured CUDA graph. */
 int tncb_plan_create(tncb_ctx* ctx, const tncb_tn* tn, const tncb_path* path, tncb_plan** out);
+/* A plan in a chosen element type: execute / stage / run / stage_slices / run_slices then work in that type (the static
+ * layout, batch descriptors and workspace limits use its element size; tncb_plan_info reports bytes at it). */
+int tncb_plan_create_dt(tncb_ctx* ctx, const tncb_tn* tn, const tncb_path* path, int dtype, tncb_plan** out);
 /* `tn` must have the structure the plan was compiled from: every leaf is re-validated (kind, rank,
  * dims, non-null payload, live device handle) -> TNCB_ERR_INVALID / TNCB_ERR_SHAPE /
  * TNCB_ERR_UNCONTRACTED before any copy.  Device leaves: same atomic rule as above.  A plan may be
@@ -286,7 +317,8 @@ int tncb_plan_run(tncb_ctx* ctx, tncb_plan* plan, tncb_tensor** out, int* n_out,
 int tncb_plan_stage_slices(tncb_ctx* ctx, tncb_plan* plan, size_t n_slices, const tncb_tn* const* slice_tns);
 int tncb_plan_run_slices(tncb_ctx* ctx, tncb_plan* plan, size_t first, size_t stride,
                          tncb_tensor** out_sum, int* n_out, uint64_t* out_legs);
-/* Schedule facts: #pairs, sum 8MNK, sum 16(MK+KN+MN), peak arena bytes, #kernels. */
+/* Schedule facts: #pairs, sum 8MNK, sum s(MK+KN+MN), peak arena bytes, #kernels (s = 16 B per element for complex128,
+ * 8 B for complex64 plans). */
 int tncb_plan_info(const tncb_plan* plan, uint64_t* n_pairs, double* flops, double* bytes,
                    uint64_t* peak_bytes, uint64_t* n_kernels);
 void tncb_plan_destroy(tncb_plan* plan);
@@ -330,6 +362,7 @@ int tncb_hdf5_store(const char* path, size_t n, const char* const* names, const 
 /* 128-byte NCCL unique id; create on rank 0, broadcast out of band. */
 int tncb_comm_unique_id(uint8_t id_out[128]);
 int tncb_comm_init(tncb_ctx* ctx, int world_size, int rank, const uint8_t id[128]);
+/* send / recv / allreduce_sum move complex128 tensors only: a complex64 tensor -> TNCB_ERR_UNSUPPORTED. */
 int tncb_comm_send(tncb_ctx* ctx, const tncb_tensor* t, int peer);
 int tncb_comm_recv(tncb_ctx* ctx, int rank_dims, const uint64_t* dims, int peer, tncb_tensor** out);
 /* In-place sum over all ranks (ncclAllReduce on the ctx stream): combines sliced contractions. */

@@ -14,9 +14,20 @@ from typing import Sequence
 
 import numpy as np
 
-from ._lib import TncbError, check, lib, u64_array
+from ._lib import TNCB_C64, TNCB_C128, TncbError, check, lib, u64_array
 
-__all__ = ["Context", "DeviceTensor", "TncbError", "contract_pair", "contract_pair_into", "default_context", "lib"]
+__all__ = ["Context", "DeviceTensor", "TncbError", "contract_pair", "contract_pair_into", "default_context", "dtype_code", "lib"]
+
+_DTYPE_CODES = {np.dtype(np.complex128): TNCB_C128, np.dtype(np.complex64): TNCB_C64}
+_CODE_DTYPES = {v: k for k, v in _DTYPE_CODES.items()}
+
+
+def dtype_code(dtype) -> int:
+    """tncb_dtype of numpy.complex128 / numpy.complex64; any other dtype raises ValueError (before any library call)."""
+    try:
+        return _DTYPE_CODES[np.dtype(dtype)]
+    except (TypeError, KeyError):
+        raise ValueError(f"dtype must be numpy.complex128 or numpy.complex64, got {dtype!r}") from None
 
 
 class Context:
@@ -125,25 +136,29 @@ def default_context() -> Context:
 
 
 class DeviceTensor:
-    """A device-resident complex128 tensor (tncb_tensor), row-major."""
+    """A device-resident complex128 or complex64 tensor (tncb_tensor), row-major."""
 
-    def __init__(self, ctx: Context, handle, shape: Sequence[int]):
+    def __init__(self, ctx: Context, handle, shape: Sequence[int], dtype=np.complex128):
         self.ctx = ctx
         self.handle = handle
         self.shape = tuple(int(s) for s in shape)
+        self.dtype = np.dtype(dtype)
 
     @classmethod
-    def from_numpy(cls, ctx: Context, arr: np.ndarray) -> "DeviceTensor":
-        a = np.asarray(arr, dtype=np.complex128, order="C")  # (ascontiguousarray would promote 0-d to 1-d)
+    def from_numpy(cls, ctx: Context, arr: np.ndarray, dtype=np.complex128) -> "DeviceTensor":
+        """Upload `arr` converted to `dtype` (complex128 unless complex64 is asked for explicitly)."""
+        code = dtype_code(dtype)
+        a = np.asarray(arr, dtype=dtype, order="C")  # (ascontiguousarray would promote 0-d to 1-d)
         h = C.c_void_p()
-        check(ctx._l.tncb_tensor_upload(ctx.handle, a.ndim, u64_array(a.shape), a.ctypes.data_as(C.c_void_p), C.byref(h)))
-        return cls(ctx, h, a.shape)
+        check(ctx._l.tncb_tensor_upload_dt(ctx.handle, a.ndim, u64_array(a.shape), code, a.ctypes.data_as(C.c_void_p), C.byref(h)))
+        return cls(ctx, h, a.shape, dtype)
 
     @classmethod
-    def empty(cls, ctx: Context, shape: Sequence[int]) -> "DeviceTensor":
+    def empty(cls, ctx: Context, shape: Sequence[int], dtype=np.complex128) -> "DeviceTensor":
+        code = dtype_code(dtype)
         h = C.c_void_p()
-        check(ctx._l.tncb_tensor_alloc(ctx.handle, len(shape), u64_array(shape), C.byref(h)))
-        return cls(ctx, h, shape)
+        check(ctx._l.tncb_tensor_alloc_dt(ctx.handle, len(shape), u64_array(shape), code, C.byref(h)))
+        return cls(ctx, h, shape, dtype)
 
     @classmethod
     def adopt(cls, ctx: Context, handle) -> "DeviceTensor":
@@ -151,12 +166,13 @@ class DeviceTensor:
         r = l.tncb_tensor_rank(handle)
         dims = u64_array([0] * max(r, 1))
         check(l.tncb_tensor_dims(handle, dims))
-        return cls(ctx, handle, [dims[i] for i in range(r)])
+        return cls(ctx, handle, [dims[i] for i in range(r)], _CODE_DTYPES[l.tncb_tensor_dtype(handle)])
 
     def to_numpy(self) -> np.ndarray:
+        """A host copy in the tensor's own dtype."""
         if self.handle is None:
             raise TncbError(-3, "Cannot convert uncontracted tensor to data")
-        out = np.empty(self.shape, dtype=np.complex128)
+        out = np.empty(self.shape, dtype=self.dtype)
         check(self.ctx._l.tncb_tensor_download(self.ctx.handle, self.handle, out.ctypes.data_as(C.c_void_p)))
         return out
 

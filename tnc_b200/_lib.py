@@ -80,6 +80,9 @@ SIGNATURES = {
     "tncb_ctx_last_gemm_ms": (C.c_int, [C.c_void_p, C.POINTER(C.c_float)]),
     "tncb_tensor_upload": (C.c_int, [C.c_void_p, C.c_int, u64p, C.c_void_p, vpp]),
     "tncb_tensor_alloc": (C.c_int, [C.c_void_p, C.c_int, u64p, vpp]),
+    "tncb_tensor_upload_dt": (C.c_int, [C.c_void_p, C.c_int, u64p, C.c_int, C.c_void_p, vpp]),
+    "tncb_tensor_alloc_dt": (C.c_int, [C.c_void_p, C.c_int, u64p, C.c_int, vpp]),
+    "tncb_tensor_dtype": (C.c_int, [C.c_void_p]),
     "tncb_tensor_download": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "tncb_tensor_write": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "tncb_tensor_read": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -99,8 +102,10 @@ SIGNATURES = {
     "tncb_tensor_add": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "tncb_gate_matrix": (C.c_int, [C.c_char_p, f64p, C.c_int, C.c_int, f64p, i32p]),
     "tncb_contract_tensor_network": (C.c_int, [C.c_void_p, C.POINTER(TncbTn), C.POINTER(TncbPath), vpp, i32p, u64p]),
+    "tncb_contract_tensor_network_dt": (C.c_int, [C.c_void_p, C.POINTER(TncbTn), C.POINTER(TncbPath), C.c_int, vpp, i32p, u64p]),
     "tncb_network_out_legs": (C.c_int, [C.POINTER(TncbTn), C.POINTER(TncbPath), i32p, u64p, u64p]),
     "tncb_plan_create": (C.c_int, [C.c_void_p, C.POINTER(TncbTn), C.POINTER(TncbPath), vpp]),
+    "tncb_plan_create_dt": (C.c_int, [C.c_void_p, C.POINTER(TncbTn), C.POINTER(TncbPath), C.c_int, vpp]),
     "tncb_plan_execute": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(TncbTn), vpp, i32p, u64p]),
     "tncb_plan_stage": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(TncbTn)]),
     "tncb_plan_run": (C.c_int, [C.c_void_p, C.c_void_p, vpp, i32p, u64p]),
@@ -127,6 +132,10 @@ SIGNATURES = {
     "tncb_hdf5_store": (C.c_int, [C.c_char_p, C.c_size_t, C.POINTER(C.c_char_p), C.POINTER(C.c_int), C.POINTER(u64p),
                                   C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.POINTER(u64p)]),
 }
+
+# tncb_dtype values
+TNCB_C128 = 0
+TNCB_C64 = 1
 
 _lib = None
 

@@ -155,18 +155,22 @@ class SlicedPlan:
     """Compile + stage once, run many: the sliced contraction with every slice's leaf block resident on the device and
     the slice loop inside libtncb200 (tncb_plan_stage_slices / tncb_plan_run_slices)."""
 
-    def __init__(self, tn: Tensor, path: ContractionPath, legs: Sequence[int], ctx=None):
-        from .. import default_context
+    def __init__(self, tn: Tensor, path: ContractionPath, legs: Sequence[int], ctx=None, dtype=np.complex128):
+        from .. import default_context, dtype_code
         from ..tensornetwork.contraction import NetworkPlan
+        dtype_code(dtype)
+        self.dtype = np.dtype(dtype)
         self.ctx = ctx or default_context()
         self.sn = SlicedNetwork(tn, legs)
         nets = [self.sn.slice(a) for a in self.sn.assignments]
         self.n_slices = len(nets)
-        self.plan = NetworkPlan(nets[0], path, ctx=self.ctx)
+        self.plan = NetworkPlan(nets[0], path, ctx=self.ctx, dtype=dtype)
         self.plan.stage_slices(nets)
 
     def run(self, rank: int = 0, world: int = 1, allreduce: bool = True) -> Tensor:
         from .._lib import check
+        if world > 1 and self.dtype == np.complex64:
+            raise ValueError("multi-rank sliced runs are complex128 only (the NCCL all-reduce has no complex64 path)")
         total = self.plan.run_slices(rank, world)
         if world > 1 and allreduce:
             check(self.ctx._l.tncb_comm_allreduce_sum(self.ctx.handle, total.tensordata.matrix.handle))
@@ -174,9 +178,13 @@ class SlicedPlan:
 
 
 def contract_sliced(tn: Tensor, path: ContractionPath, legs: Sequence[int], ctx=None, rank: int = 0, world: int = 1,
-                    allreduce: bool = True) -> Tensor:
+                    allreduce: bool = True, dtype=np.complex128) -> Tensor:
     """Contracts every slice assigned to this rank (round-robin: slices rank, rank + world, ...), accumulates on the
     device and, with world > 1, sums over ranks with one NCCL all-reduce (`tncb_comm_allreduce_sum`; the communicator must
     have been set up with `dist.init_device_comm`).  One schedule is compiled, all slice payloads are uploaded once and
-    the slice loop runs inside the library; `SlicedPlan` keeps that state for repeated runs."""
-    return SlicedPlan(tn, path, legs, ctx).run(rank, world, allreduce)
+    the slice loop runs inside the library; `SlicedPlan` keeps that state for repeated runs.  dtype=np.complex64 runs
+    the slices in complex64 (single rank only)."""
+    from .. import TNCB_C64, dtype_code
+    if world > 1 and dtype_code(dtype) == TNCB_C64:      # refused before any slice is staged
+        raise ValueError("multi-rank sliced runs are complex128 only (the NCCL all-reduce has no complex64 path)")
+    return SlicedPlan(tn, path, legs, ctx, dtype).run(rank, world, allreduce)

@@ -103,6 +103,7 @@ int tncb_comm_init(tncb_ctx* ctx, int world_size, int rank, const uint8_t id_in[
 
 int tncb_comm_send(tncb_ctx* ctx, const tncb_tensor* t, int peer) {
   if (!ctx || !t) return fail(TNCB_ERR_INVALID, "null argument");
+  if (t->dtype != TNCB_C128) return fail(TNCB_ERR_UNSUPPORTED, "NCCL transfers of complex64 tensors are not supported");
   if (!ctx->nccl_comm) return fail(TNCB_ERR_NCCL, "communicator not initialised");
   TNCB_CUDA(cudaSetDevice(ctx->device));
   TNCB_NCCL(g_nccl.Send(t->ptr, (size_t)t->elems * 2, kNcclFloat64, peer, ctx->nccl_comm, ctx->stream));
@@ -124,6 +125,7 @@ int tncb_comm_recv(tncb_ctx* ctx, int rank_dims, const uint64_t* dims, int peer,
 
 int tncb_comm_allreduce_sum(tncb_ctx* ctx, tncb_tensor* t) {
   if (!ctx || !t) return fail(TNCB_ERR_INVALID, "null argument");
+  if (t->dtype != TNCB_C128) return fail(TNCB_ERR_UNSUPPORTED, "NCCL transfers of complex64 tensors are not supported");
   if (!ctx->nccl_comm) return fail(TNCB_ERR_NCCL, "communicator not initialised");
   TNCB_CUDA(cudaSetDevice(ctx->device));
   TNCB_NCCL(g_nccl.AllReduce(t->ptr, t->ptr, (size_t)t->elems * 2, kNcclFloat64, /*ncclSum*/ 0, ctx->nccl_comm, ctx->stream));

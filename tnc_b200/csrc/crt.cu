@@ -165,8 +165,13 @@ __device__ __forceinline__ void crt_tile_coord(int e, int lk, int& r, int& k) {
   r = (rb << (5 - lk)) + (lane >> lk);
 }
 
+// complex64 operands (E = float2) are widened exactly to f64 as they are loaded, in this kernel and the residue kernel.
+__device__ __forceinline__ double2 crt_ld(const double2* p) { return __ldg(p); }
+__device__ __forceinline__ double2 crt_ld(const float2* p) { const float2 v = __ldg(p); return make_double2((double)v.x, (double)v.y); }
+
+template <typename E>
 __global__ void __launch_bounds__(256)
-crt_rowmax_kernel(const double2* __restrict__ src, const long long* __restrict__ off_row, const long long* __restrict__ off_k,
+crt_rowmax_kernel(const E* __restrict__ src, const long long* __restrict__ off_row, const long long* __restrict__ off_k,
                   long long rows, long long K, int lk, unsigned long long* __restrict__ rowmax) {
   __shared__ unsigned long long s_max[RES_ROWS_C];
   __shared__ long long s_offr[RES_ROWS_C], s_offk[RES_K_C];
@@ -184,7 +189,7 @@ crt_rowmax_kernel(const double2* __restrict__ src, const long long* __restrict__
     const long long orow = s_offr[r], ok = s_offk[k];
     mv[it] = 0ull;
     if (orow >= 0 && ok >= 0) {
-      const double2 v = __ldg(src + orow + ok);
+      const double2 v = crt_ld(src + orow + ok);
       mv[it] = max((unsigned long long)__double_as_longlong(fabs(v.x)), (unsigned long long)__double_as_longlong(fabs(v.y)));
     }
   }
@@ -225,9 +230,9 @@ __device__ __forceinline__ int crt_fix_byte(int s, int m) {
   return s;
 }
 constexpr int RES_ROWS = RES_ROWS_C, RES_K = RES_K_C, RES_RS = RES_K + RES_K / 8 + 1;   // padded row stride (elements)
-template <int COMPS, bool KARA>
+template <int COMPS, bool KARA, typename E>
 __global__ void __launch_bounds__(256, 3)
-crt_residue_kernel(const double2* __restrict__ src, const long long* __restrict__ off_row, const long long* __restrict__ off_k,
+crt_residue_kernel(const E* __restrict__ src, const long long* __restrict__ off_row, const long long* __restrict__ off_k,
                    long long rows, long long K, long long rowsP, long long Kp, const unsigned long long* __restrict__ rowmax, int bits, int lk,
                    const __grid_constant__ CrtTables T, int8_t* __restrict__ planes) {
   extern __shared__ __align__(16) unsigned char res_smem_raw[];
@@ -258,7 +263,7 @@ crt_residue_kernel(const double2* __restrict__ src, const long long* __restrict_
     crt_tile_coord(it * 256 + tid, lk, r, k);
     const long long orow = s_offr[r], ok = s_offk[k];
     vv[it] = make_double2(0.0, 0.0);
-    if (orow >= 0 && ok >= 0) vv[it] = __ldg(src + orow + ok);
+    if (orow >= 0 && ok >= 0) vv[it] = crt_ld(src + orow + ok);
   }
 #pragma unroll
   for (int it = 0; it < RES_ROWS * RES_K / 256; it++) {
@@ -592,7 +597,7 @@ crt_gemm_kernel(const __grid_constant__ CUtensorMap mapB, const __grid_constant_
 // ---- CRT reconstruction -------------------------------------------------------------------------------
 struct CrtReconArgs {
   const int8_t* R;
-  double2* C;          // &C[n_begin * ldc + m_begin]
+  void* C;             // &C[n_begin * ldc + m_begin]: double2, or float2 for complex64 pairs
   const unsigned long long* max_n;   // row maxima (bit patterns) of this panel's Bt rows
   const unsigned long long* max_m;   // ... of this panel's At rows
   long long rows, cols, ldc;   // valid panel extent, row stride of C
@@ -606,7 +611,7 @@ struct CrtReconArgs {
 // mantissa word, one DADD removes 2^52 + 128 nkc.
 // KARA (three products): the planes hold k1, k2, k3 (+128 each); re = k1 - k2 and im = k3 - k1 - k2 are formed here from the
 // bytes (the CRT sum is linear, no reduction mod m_i needed: |y| <= 3 * 128 * 32 < 2^13.6 keeps S1 exact, 13.6 + 34 + 4.4 bits).
-template <bool ONE_CHUNK, bool KARA>
+template <bool ONE_CHUNK, bool KARA, typename TO>
 __global__ void __launch_bounds__(256, 4)
 crt_reconstruct_kernel(const __grid_constant__ CrtReconArgs a, const __grid_constant__ CrtTables T) {
   const long long cols4 = a.Mp >> 2;
@@ -667,7 +672,7 @@ crt_reconstruct_kernel(const __grid_constant__ CrtReconArgs a, const __grid_cons
     }
   }
   const int en = crt_exp_from_bits(a.max_n[n]);
-  double2* dst = a.C + n * a.ldc + m4;
+  TO* dst = static_cast<TO*>(a.C) + n * a.ldc + m4;
   const double RMAGIC = 6755399441055744.0;
 #pragma unroll
   for (int j = 0; j < 4; j++) {
@@ -683,7 +688,8 @@ crt_reconstruct_kernel(const __grid_constant__ CrtReconArgs a, const __grid_cons
       const double fr = (s1r[j] - qr) + s2r[j], fi = (s1i[j] - qi) + s2i[j];
       out = make_double2(scalbn(fr * T.p_scaled, en + em), scalbn(fi * T.p_scaled, en + em));
     }
-    dst[j] = out;
+    if constexpr (sizeof(TO) == sizeof(double2)) dst[j] = out;
+    else dst[j] = make_float2((float)out.x, (float)out.y);   // the one rounding of a complex64 result
   }
 }
 
@@ -719,10 +725,14 @@ static inline long long round_up_ll(long long x, long long a) { return (x + a - 
 
 
 // tables: offAm[M], offBn[N], offAk[K], offBk[K] (built by the caller, see kernels.cu)
-int launch_k1_crt(tncb_ctx* ctx, const PairPlan& P, const double2* A, const double2* B, double2* C,
-                  const long long* offAm, const long long* offBn, const long long* offAk, const long long* offBk) {
+template <typename E>
+static int launch_k1_crt_t(tncb_ctx* ctx, const PairPlan& P, const E* A, const E* B, E* C,
+                           const long long* offAm, const long long* offBn, const long long* offAk, const long long* offBk) {
   int nmod, bits_a, bits_b;
-  const int want = ctx->crt_tol > 0.0 ? crt_bits_for_tolerance(P.K, ctx->crt_tol) : ctx->crt_bits;
+  // complex64 operands carry 24-bit mantissas: a = 28 bits keep the bound at 2^-24 K max|b| max|a|, the worst case of an
+  // FP32 dot product, with about 9 instead of 16 moduli at K = 4096.  A tolerance set on the context still decides.
+  const int dflt = sizeof(E) == sizeof(double2) ? ctx->crt_bits : kCrtBitsC64;
+  const int want = ctx->crt_tol > 0.0 ? crt_bits_for_tolerance(P.K, ctx->crt_tol) : dflt;
   crt_choose(P.K, want, ctx->crt_nmod_force, &nmod, &bits_a, &bits_b);
   CrtTables T;
   crt_make_tables(nmod, bits_a, bits_b, T);
@@ -777,14 +787,14 @@ int launch_k1_crt(tncb_ctx* ctx, const PairPlan& P, const double2* A, const doub
   static bool attr_done_dev[64] = {false};          // cudaFuncSetAttribute is per device
   bool& attr_done = attr_done_dev[ctx->device & 63];
   const int smem_gemm = CRT_RING_BYTES + 8 * CRT_STG_BYTES + 1024;
-  const int smem_res = RES_ROWS * RES_RS * (int)sizeof(double2);
+  const int smem_res = RES_ROWS * RES_RS * (int)sizeof(double2);   // (the tile holds widened, truncated values)
   if (!attr_done) {
     cudaError_t e = cudaFuncSetAttribute(crt_gemm_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_gemm);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(crt_gemm_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_gemm);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(crt_residue_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_res);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(crt_residue_kernel<3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_res);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(crt_residue_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_res);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(crt_residue_kernel<3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_res);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(crt_residue_kernel<2, false, E>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_res);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(crt_residue_kernel<3, false, E>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_res);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(crt_residue_kernel<2, true, E>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_res);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(crt_residue_kernel<3, true, E>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_res);
     if (e != cudaSuccess) { cleanup(); return fail(TNCB_ERR_CUDA, cudaGetErrorString(e)); }
     attr_done = true;
   }
@@ -811,8 +821,8 @@ int launch_k1_crt(tncb_ctx* ctx, const PairPlan& P, const double2* A, const doub
     {
       dim3 g((unsigned)((nrows + RES_ROWS - 1) / RES_ROWS), (unsigned)(Kp / RES_K));
       crt_rowmax_kernel<<<g, 256, 0, st>>>(B, offBn + n0, offBk, nrows, P.K, lk_b, max_n);
-      if (kara) crt_residue_kernel<2, true><<<g, 256, smem_res, st>>>(B, offBn + n0, offBk, nrows, P.K, Np, Kp, max_n, bits_b, lk_b, T, (int8_t*)pb);
-      else crt_residue_kernel<2, false><<<g, 256, smem_res, st>>>(B, offBn + n0, offBk, nrows, P.K, Np, Kp, max_n, bits_b, lk_b, T, (int8_t*)pb);
+      if (kara) crt_residue_kernel<2, true, E><<<g, 256, smem_res, st>>>(B, offBn + n0, offBk, nrows, P.K, Np, Kp, max_n, bits_b, lk_b, T, (int8_t*)pb);
+      else crt_residue_kernel<2, false, E><<<g, 256, smem_res, st>>>(B, offBn + n0, offBk, nrows, P.K, Np, Kp, max_n, bits_b, lk_b, T, (int8_t*)pb);
     }
     ctx->launches += 2;
     CUtensorMap mapB;
@@ -825,8 +835,8 @@ int launch_k1_crt(tncb_ctx* ctx, const PairPlan& P, const double2* A, const doub
       {
         dim3 g((unsigned)((mcols + RES_ROWS - 1) / RES_ROWS), (unsigned)(Kp / RES_K));
         crt_rowmax_kernel<<<g, 256, 0, st>>>(A, offAm + m0, offAk, mcols, P.K, lk_a, max_m);
-        if (kara) crt_residue_kernel<3, true><<<g, 256, smem_res, st>>>(A, offAm + m0, offAk, mcols, P.K, Mp, Kp, max_m, bits_a, lk_a, T, (int8_t*)pa);
-        else crt_residue_kernel<3, false><<<g, 256, smem_res, st>>>(A, offAm + m0, offAk, mcols, P.K, Mp, Kp, max_m, bits_a, lk_a, T, (int8_t*)pa);
+        if (kara) crt_residue_kernel<3, true, E><<<g, 256, smem_res, st>>>(A, offAm + m0, offAk, mcols, P.K, Mp, Kp, max_m, bits_a, lk_a, T, (int8_t*)pa);
+        else crt_residue_kernel<3, false, E><<<g, 256, smem_res, st>>>(A, offAm + m0, offAk, mcols, P.K, Mp, Kp, max_m, bits_a, lk_a, T, (int8_t*)pa);
       }
       ctx->launches += 2;
       CUtensorMap mapA;
@@ -862,11 +872,11 @@ int launch_k1_crt(tncb_ctx* ctx, const PairPlan& P, const double2* A, const doub
       const long long threads = nrows * (Mp / 4);
       const unsigned rg = (unsigned)((threads + 255) / 256);
       if (kara) {
-        if (nkc == 1) crt_reconstruct_kernel<true, true><<<rg, 256, 0, st>>>(r, T);
-        else crt_reconstruct_kernel<false, true><<<rg, 256, 0, st>>>(r, T);
+        if (nkc == 1) crt_reconstruct_kernel<true, true, E><<<rg, 256, 0, st>>>(r, T);
+        else crt_reconstruct_kernel<false, true, E><<<rg, 256, 0, st>>>(r, T);
       } else {
-        if (nkc == 1) crt_reconstruct_kernel<true, false><<<rg, 256, 0, st>>>(r, T);
-        else crt_reconstruct_kernel<false, false><<<rg, 256, 0, st>>>(r, T);
+        if (nkc == 1) crt_reconstruct_kernel<true, false, E><<<rg, 256, 0, st>>>(r, T);
+        else crt_reconstruct_kernel<false, false, E><<<rg, 256, 0, st>>>(r, T);
       }
       ctx->launches += 2;
     }
@@ -876,6 +886,13 @@ int launch_k1_crt(tncb_ctx* ctx, const PairPlan& P, const double2* A, const doub
   cleanup();   // stream-ordered reuse: later allocations are only touched by later kernels
   if (e != cudaSuccess) return fail(TNCB_ERR_CUDA, std::string("K1' (CRT) launch: ") + cudaGetErrorString(e));
   return TNCB_OK;
+}
+
+int launch_k1_crt(tncb_ctx* ctx, const PairPlan& P, const void* A, const void* B, void* C,
+                  const long long* offAm, const long long* offBn, const long long* offAk, const long long* offBk, int dtype) {
+  if (dtype == TNCB_C64)
+    return launch_k1_crt_t(ctx, P, (const float2*)A, (const float2*)B, (float2*)C, offAm, offBn, offAk, offBk);
+  return launch_k1_crt_t(ctx, P, (const double2*)A, (const double2*)B, (double2*)C, offAm, offBn, offAk, offBk);
 }
 
 } // namespace tncb

@@ -62,8 +62,9 @@ struct Arena {
 } // namespace tncb
 
 struct tncb_tensor {
-  double2* ptr = nullptr;
+  double2* ptr = nullptr;   // float2 data for TNCB_C64 (see dtype)
   int rank = 0;
+  int dtype = TNCB_C128;
   uint64_t dims[tncb::kMaxLegs];
   uint64_t elems = 1;
   size_t bytes = 0;      // arena bytes (0 = not owned by the arena)
@@ -120,20 +121,27 @@ struct tncb_ctx {
 extern "C" void tncb_plan_release_device_state(struct tncb_plan* plan);
 
 namespace tncb {
+// bytes per element of a tncb_dtype (0: not a dtype)
+inline size_t dtype_size(int dtype) { return dtype == TNCB_C128 ? 16 : dtype == TNCB_C64 ? 8 : 0; }
+
 // ---- kernel launchers (kernels.cu) ---------------------------------------------------
-int launch_pair(tncb_ctx* ctx, const PairPlan& p, const double2* A, const double2* B, double2* C);
-int launch_permute(tncb_ctx* ctx, const double2* in, double2* out, int rank,
-                   const uint64_t* in_dims, const int* perm);
-int launch_conj(tncb_ctx* ctx, double2* data, uint64_t elems);
-int launch_add(tncb_ctx* ctx, double2* dst, const double2* src, uint64_t elems);
+// Operands and results are complex128 (double2) or, for dtype TNCB_C64, complex64 (float2); split-K partials are
+// double2 for both.  Kernel and configuration choices never depend on the dtype.
+int launch_pair(tncb_ctx* ctx, const PairPlan& p, const void* A, const void* B, void* C, int dtype = TNCB_C128);
+int launch_permute(tncb_ctx* ctx, const void* in, void* out, int rank,
+                   const uint64_t* in_dims, const int* perm, int dtype = TNCB_C128);
+int launch_conj(tncb_ctx* ctx, void* data, uint64_t elems, int dtype = TNCB_C128);
+int launch_add(tncb_ctx* ctx, void* dst, const void* src, uint64_t elems, int dtype = TNCB_C128);
 int ensure_tab(tncb_ctx* ctx, size_t elems);
 // K1': tcgen05 int8-sliced ZGEMM (ozaki.cu); tables as built by launch_k1
 int launch_k1_ozaki(tncb_ctx* ctx, const PairPlan& p, const double2* A, const double2* B, double2* C, int S,
                     const long long* offAm, const long long* offBn, const long long* offAk, const long long* offBk);
 
 // K1' default engine: tcgen05 int8 GEMMs over coprime moduli + CRT reconstruction (crt.cu)
-int launch_k1_crt(tncb_ctx* ctx, const PairPlan& p, const double2* A, const double2* B, double2* C,
-                  const long long* offAm, const long long* offBn, const long long* offAk, const long long* offBk);
+int launch_k1_crt(tncb_ctx* ctx, const PairPlan& p, const void* A, const void* B, void* C,
+                  const long long* offAm, const long long* offBn, const long long* offAk, const long long* offBk,
+                  int dtype = TNCB_C128);
+constexpr int kCrtBitsC64 = 28;   // default operand bits of complex64 pairs: bound 2^-24 K max|b[n,:]| max|a[m,:]|
 void crt_choose(long long K, int want_bits, int nmod_force, int* nmod, int* bits_a, int* bits_b);
 int crt_bits_for_tolerance(long long K, double tol);
 int crt_export_tables(int nmod, int* moduli, double* rho1, double* rho2, double* log2_product);
@@ -155,9 +163,10 @@ struct K0BatchItem {
 };
 bool k0_batch_eligible(int sm_count, const PairPlan& p);
 int k0_batch_fill(int sm_count, const PairPlan& p, K0BatchItem* item);   // returns the number of 256-thread blocks of the item
-int launch_k0_batch(tncb_ctx* ctx, const K0BatchItem* d_items, const int* d_block_start, int n_items, int total_blocks, char* ws);
+int launch_k0_batch(tncb_ctx* ctx, const K0BatchItem* d_items, const int* d_block_start, int n_items, int total_blocks, char* ws,
+                    int dtype = TNCB_C128);
 
-int tensor_new(tncb_ctx* ctx, int rank, const uint64_t* dims, tncb_tensor** out);
+int tensor_new(tncb_ctx* ctx, int rank, const uint64_t* dims, tncb_tensor** out, int dtype = TNCB_C128);
 
 // TensorData::File leaf (hdf5io.cpp): first member of /tensors, optionally adjointed, checked against the leaf's dims
 namespace h5 { int load_file_leaf(const char* path, bool adjoint, int rank, const uint64_t* dims, double* out_re_im); }

@@ -13,6 +13,11 @@
 //       ring, FP64 tensor-core DMMA (mma.sync.m8n8k4.f64, 4 real MMAs per complex tile).
 //       tcgen05.mma has no f64 kind, so the FP64 tensor path on sm_100a is DMMA; measured
 //       peak 37.2 TFLOP/s (profiles/r01_fp64_peak_microbench.txt).
+//
+// complex64 (TNCB_C64): every kernel has a float2 instantiation that reads the 8-byte operands, widens them exactly to
+// f64, runs the f64 arithmetic of the complex128 kernel in the same order and rounds once at the final store (split-K
+// partials stay f64).  Launch configurations are chosen from the pair alone, so the complex64 result is bit for bit
+// complex64(complex128 kernel(widen(a), widen(b))).
 #include "internal.h"
 #include <algorithm>
 #include <cstdio>
@@ -36,6 +41,16 @@ struct NvtxPairRange {
   }
   ~NvtxPairRange() { if (on) nvtxRangePop(); }
 };
+
+// ------------------------------------------------------------------------------------------
+// element access: load + exact widening to f64, one rounding at the store
+// ------------------------------------------------------------------------------------------
+__device__ __forceinline__ double2 widen(const double2 v) { return v; }
+__device__ __forceinline__ double2 widen(const float2 v) { return make_double2((double)v.x, (double)v.y); }
+template <typename T>
+__device__ __forceinline__ double2 ldg_wide(const T* p) { return widen(__ldg(p)); }
+__device__ __forceinline__ void st_round(double2* p, double x, double y) { *p = make_double2(x, y); }
+__device__ __forceinline__ void st_round(float2* p, double x, double y) { *p = make_float2((float)x, (float)y); }
 
 // ------------------------------------------------------------------------------------------
 // index helpers
@@ -78,9 +93,10 @@ struct K0Args {
 constexpr int K0_THREADS = 256;
 constexpr int K0_KT = 1024;
 
-template <int G>
+// T: operand type, TO: output type (double2 for split-K partials)
+template <int G, typename T, typename TO>
 __global__ void __launch_bounds__(K0_THREADS)
-k0_kernel(const double2* __restrict__ A, const double2* __restrict__ B, double2* __restrict__ dst,
+k0_kernel(const T* __restrict__ A, const T* __restrict__ B, TO* __restrict__ dst,
           const __grid_constant__ K0Args p) {
   __shared__ long long s_ka[K0_KT];
   __shared__ long long s_kb[K0_KT];
@@ -108,8 +124,8 @@ k0_kernel(const double2* __restrict__ A, const double2* __restrict__ B, double2*
     if (valid) {
 #pragma unroll 4
       for (int i = lane_g; i < cnt; i += G) {
-        const double2 a = __ldg(A + offA0 + s_ka[i]);
-        const double2 b = __ldg(B + offB0 + s_kb[i]);
+        const double2 a = ldg_wide(A + offA0 + s_ka[i]);
+        const double2 b = ldg_wide(B + offB0 + s_kb[i]);
         cr = fma(b.x, a.x, cr); cr = fma(-b.y, a.y, cr);
         ci = fma(b.x, a.y, ci); ci = fma(b.y, a.x, ci);
       }
@@ -120,16 +136,17 @@ k0_kernel(const double2* __restrict__ A, const double2* __restrict__ B, double2*
     cr += __shfl_xor_sync(0xffffffffu, cr, d);
     ci += __shfl_xor_sync(0xffffffffu, ci, d);
   }
-  if (valid && lane_g == 0) dst[(long long)blockIdx.y * MN + o] = make_double2(cr, ci);
+  if (valid && lane_g == 0) st_round(dst + (long long)blockIdx.y * MN + o, cr, ci);
 }
 
-__global__ void reduce_partials_kernel(const double2* __restrict__ part, double2* __restrict__ C,
+template <typename TO>
+__global__ void reduce_partials_kernel(const double2* __restrict__ part, TO* __restrict__ C,
                                        long long MN, int ksplit) {
   long long o = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (o >= MN) return;
   double cr = 0.0, ci = 0.0;
   for (int s = 0; s < ksplit; s++) { double2 v = part[(long long)s * MN + o]; cr += v.x; ci += v.y; }
-  C[o] = make_double2(cr, ci);
+  st_round(C + o, cr, ci);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -151,6 +168,16 @@ __device__ __forceinline__ void cp_async16(unsigned smem_addr, const void* gptr,
   const int src = pred ? 16 : 0;
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(smem_addr), "l"(gptr), "r"(src));
 }
+// complex64 operands: 8-byte gathers (.cg only takes 16 bytes)
+__device__ __forceinline__ void cp_async8(unsigned smem_addr, const void* gptr, bool pred) {
+  const int src = pred ? 8 : 0;
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;\n" ::"r"(smem_addr), "l"(gptr), "r"(src));
+}
+template <typename T>
+__device__ __forceinline__ void cp_async_elem(unsigned smem_addr, const T* gptr, bool pred) {
+  if constexpr (sizeof(T) == 16) cp_async16(smem_addr, gptr, pred);
+  else cp_async8(smem_addr, gptr, pred);
+}
 // volatile so that ptxas keeps the load where it is written (it otherwise sinks the prefetch to
 // its first use and the latency reappears as a long_scoreboard stall in the gather issue)
 __device__ __forceinline__ long long ldg_pinned(const long long* p) {
@@ -171,9 +198,9 @@ __device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double
 constexpr int K1_BK = 16;
 
 struct K1Args {
-  const double2* A;
-  const double2* B;
-  double2* C;
+  const void* A;        // double2 (complex128) or float2 (complex64) operands
+  const void* B;
+  void* C;              // complex128: double2; complex64: float2, or double2 partials when ksplit > 1
   const long long* offAm;
   const long long* offBn;
   const long long* offAk;
@@ -197,7 +224,10 @@ struct K1Args {
 // prefetched one chunk ahead into registers and the cp.async gathers of stage kc+STAGES-1 are
 // issued in the middle of chunk kc's DMMA stream, so no table load sits on the critical path
 // (ncu r01: 20 % long_scoreboard on exactly those loads before this change).
-template <int BN, int BM, int WARPS_N, int WARPS_M, int STAGES, bool B_KFAST, bool A_KFAST, int MINB = 1>
+//
+// complex64 (T = float2): the ring holds the 8-byte elements in the same fragment order (half the shared memory per
+// stage); the fragment loads widen them to f64 before the DMMAs.
+template <int BN, int BM, int WARPS_N, int WARPS_M, int STAGES, bool B_KFAST, bool A_KFAST, int MINB = 1, typename T = double2>
 __global__ void __launch_bounds__(WARPS_N* WARPS_M * 32, MINB)
 k1_kernel(const __grid_constant__ K1Args p) {
   constexpr int BK = K1_BK;
@@ -214,8 +244,11 @@ k1_kernel(const __grid_constant__ K1Args p) {
   constexpr int STAGE_ELEMS = BN * BK + BK * BM;
 
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  double2* smem = reinterpret_cast<double2*>(smem_raw);
+  T* smem = reinterpret_cast<T*>(smem_raw);
   const unsigned smem_base = (unsigned)__cvta_generic_to_shared(smem);
+  constexpr unsigned ES = sizeof(T);
+  const T* gA = static_cast<const T*>(p.A);
+  const T* gB = static_cast<const T*>(p.B);
 
   const int tid = threadIdx.x;
   const int lane = tid & 31;
@@ -289,17 +322,17 @@ k1_kernel(const __grid_constant__ K1Args p) {
     }
   };
   auto issue_stage = [&](int stage) {
-    const unsigned sbase = smem_base + (unsigned)(stage * STAGE_ELEMS) * 16u;
+    const unsigned sbase = smem_base + (unsigned)(stage * STAGE_ELEMS) * ES;
 #pragma unroll
     for (int q = 0; q < B_KO; q++)
 #pragma unroll
       for (int j = 0; j < B_ROWS; j++)
-        cp_async16(sbase + (unsigned)(b_rslot[j] + b_kslot[q]) * 16u, p.B + (b_off[j] + b_ko[q]), b_ok[j] && b_kok[q]);
+        cp_async_elem(sbase + (unsigned)(b_rslot[j] + b_kslot[q]) * ES, gB + (b_off[j] + b_ko[q]), b_ok[j] && b_kok[q]);
 #pragma unroll
     for (int q = 0; q < A_KO; q++)
 #pragma unroll
       for (int j = 0; j < A_COLS; j++)
-        cp_async16(sbase + (unsigned)(a_cslot[j] + a_kslot[q]) * 16u, p.A + (a_off[j] + a_ko[q]), a_ok[j] && a_kok[q]);
+        cp_async_elem(sbase + (unsigned)(a_cslot[j] + a_kslot[q]) * ES, gA + (a_off[j] + a_ko[q]), a_ok[j] && a_kok[q]);
   };
 
   double cr[TI][TJ][2], ci[TI][TJ][2];
@@ -319,12 +352,12 @@ k1_kernel(const __grid_constant__ K1Args p) {
   }
   if (STAGES - 1 < nk) fetch_ko(kbase + (long long)(STAGES - 1) * BK); // offsets of the first in-loop stage
 
-  auto compute_kb = [&](const double2* sB, const double2* sA, int kb) {
+  auto compute_kb = [&](const T* sB, const T* sA, int kb) {
     double2 bf[TI], af[TJ];
 #pragma unroll
-    for (int i = 0; i < TI; i++) bf[i] = sB[((wn * TI + i) * (BK / 4) + kb) * 32 + lane];
+    for (int i = 0; i < TI; i++) bf[i] = widen(sB[((wn * TI + i) * (BK / 4) + kb) * 32 + lane]);
 #pragma unroll
-    for (int j = 0; j < TJ; j++) af[j] = sA[(kb * (BM / 8) + wm * TJ + j) * 32 + lane];
+    for (int j = 0; j < TJ; j++) af[j] = widen(sA[(kb * (BM / 8) + wm * TJ + j) * 32 + lane]);
     // four passes so that the two DMMAs feeding one accumulator are TI*TJ*2 issues apart
 #pragma unroll
     for (int i = 0; i < TI; i++)
@@ -345,8 +378,8 @@ k1_kernel(const __grid_constant__ K1Args p) {
   for (int kc = 0; kc < nk; kc++) {
     cp_async_wait<STAGES - 2>();
     __syncthreads();
-    const double2* sB = smem + (kc % STAGES) * STAGE_ELEMS;
-    const double2* sA = sB + BN * BK;
+    const T* sB = smem + (kc % STAGES) * STAGE_ELEMS;
+    const T* sA = sB + BN * BK;
 #pragma unroll
     for (int kb = 0; kb < BK / 8; kb++) compute_kb(sB, sA, kb);
     {
@@ -370,9 +403,16 @@ k1_kernel(const __grid_constant__ K1Args p) {
 #pragma unroll
     for (int j = 0; j < TJ; j++) {
       const long long gm = m0 + (wm * TJ + j) * 8 + t2;
-      double2* dst = p.C + (long long)split * p.M * p.N + gn * p.M + gm;
-      if (gm < p.M) dst[0] = make_double2(cr[i][j][0], ci[i][j][0]);
-      if (gm + 1 < p.M) dst[1] = make_double2(cr[i][j][1], ci[i][j][1]);
+      const long long o = (long long)split * p.M * p.N + gn * p.M + gm;
+      if (sizeof(T) == sizeof(double2) || p.ksplit > 1) {   // complex128 result, or f64 partials
+        double2* dst = static_cast<double2*>(p.C) + o;
+        if (gm < p.M) dst[0] = make_double2(cr[i][j][0], ci[i][j][0]);
+        if (gm + 1 < p.M) dst[1] = make_double2(cr[i][j][1], ci[i][j][1]);
+      } else {
+        float2* dst = static_cast<float2*>(p.C) + o;
+        if (gm < p.M) st_round(dst, cr[i][j][0], ci[i][j][0]);
+        if (gm + 1 < p.M) st_round(dst + 1, cr[i][j][1], ci[i][j][1]);
+      }
     }
   }
 }
@@ -380,14 +420,16 @@ k1_kernel(const __grid_constant__ K1Args p) {
 // ------------------------------------------------------------------------------------------
 // permute (Permutor::apply / tetra transpose) and conjugate
 // ------------------------------------------------------------------------------------------
-__global__ void permute_kernel(const double2* __restrict__ in, double2* __restrict__ out,
+template <typename T>
+__global__ void permute_kernel(const T* __restrict__ in, T* __restrict__ out,
                                const __grid_constant__ LegList L, long long total) {
   for (long long o = (long long)blockIdx.x * blockDim.x + threadIdx.x; o < total;
        o += (long long)gridDim.x * blockDim.x)
     out[o] = __ldg(in + decomp_a(o, L));
 }
 
-__global__ void conj_kernel(double2* __restrict__ d, long long total) {
+template <typename T>
+__global__ void conj_kernel(T* __restrict__ d, long long total) {
   for (long long o = (long long)blockIdx.x * blockDim.x + threadIdx.x; o < total;
        o += (long long)gridDim.x * blockDim.x)
     d[o].y = -d[o].y;
@@ -416,9 +458,11 @@ int ensure_partial(tncb_ctx* ctx, size_t elems) {
   return TNCB_OK;
 }
 
-template <int G>
-static void launch_k0_g(dim3 grid, cudaStream_t st, const double2* A, const double2* B, double2* dst, const K0Args& a) {
-  k0_kernel<G><<<grid, K0_THREADS, 0, st>>>(A, B, dst, a);
+template <int G, typename T>
+static void launch_k0_g(dim3 grid, cudaStream_t st, const T* A, const T* B, void* dst, bool split, const K0Args& a) {
+  if constexpr (sizeof(T) == sizeof(double2)) k0_kernel<G, T, double2><<<grid, K0_THREADS, 0, st>>>(A, B, (double2*)dst, a);
+  else if (split) k0_kernel<G, T, double2><<<grid, K0_THREADS, 0, st>>>(A, B, (double2*)dst, a);
+  else k0_kernel<G, T, float2><<<grid, K0_THREADS, 0, st>>>(A, B, (float2*)dst, a);
 }
 
 // K0 launch geometry: G lanes per output, ksplit K ranges (deterministic two-pass reduction)
@@ -445,13 +489,14 @@ size_t k0_partial_elems(int sm_count, const PairPlan& P) {
   return ksplit > 1 ? (size_t)(P.M * P.N * ksplit) : 0;
 }
 
-static int launch_k0(tncb_ctx* ctx, const PairPlan& P, const double2* A, const double2* B, double2* C) {
+template <typename T>
+static int launch_k0(tncb_ctx* ctx, const PairPlan& P, const T* A, const T* B, T* C) {
   K0Args a;
   a.m = P.m; a.n = P.n; a.k = P.k; a.M = P.M; a.N = P.N; a.K = P.K;
   const long long MN = P.M * P.N;
   int G; long long ksplit;
   k0_config(ctx->sm_count, P, &G, &ksplit, &a.kchunk);
-  double2* dst = C;
+  void* dst = C;
   if (ksplit > 1) {
     if (ctx->partial_override) {   // graph capture: plan-owned scratch with a fixed address
       if ((size_t)(MN * ksplit) > ctx->partial_override_elems) return fail(TNCB_ERR_INVALID, "graph scratch too small");
@@ -466,18 +511,19 @@ static int launch_k0(tncb_ctx* ctx, const PairPlan& P, const double2* A, const d
   const long long blocks = (MN + per_block - 1) / per_block;
   if (blocks > 0x7fffffffLL) return fail(TNCB_ERR_UNSUPPORTED, "K0 grid too large");
   dim3 grid((unsigned)blocks, (unsigned)ksplit);
+  const bool split = ksplit > 1;
   switch (G) {
-    case 1: launch_k0_g<1>(grid, ctx->stream, A, B, dst, a); break;
-    case 2: launch_k0_g<2>(grid, ctx->stream, A, B, dst, a); break;
-    case 4: launch_k0_g<4>(grid, ctx->stream, A, B, dst, a); break;
-    case 8: launch_k0_g<8>(grid, ctx->stream, A, B, dst, a); break;
-    case 16: launch_k0_g<16>(grid, ctx->stream, A, B, dst, a); break;
-    default: launch_k0_g<32>(grid, ctx->stream, A, B, dst, a); break;
+    case 1: launch_k0_g<1>(grid, ctx->stream, A, B, dst, split, a); break;
+    case 2: launch_k0_g<2>(grid, ctx->stream, A, B, dst, split, a); break;
+    case 4: launch_k0_g<4>(grid, ctx->stream, A, B, dst, split, a); break;
+    case 8: launch_k0_g<8>(grid, ctx->stream, A, B, dst, split, a); break;
+    case 16: launch_k0_g<16>(grid, ctx->stream, A, B, dst, split, a); break;
+    default: launch_k0_g<32>(grid, ctx->stream, A, B, dst, split, a); break;
   }
   ctx->launches++;
   ctx->engine_count[ksplit > 1 ? 1 : 0]++;
   if (ksplit > 1) {
-    reduce_partials_kernel<<<(unsigned)((MN + 255) / 256), 256, 0, ctx->stream>>>(dst, C, MN, (int)ksplit);
+    reduce_partials_kernel<<<(unsigned)((MN + 255) / 256), 256, 0, ctx->stream>>>((const double2*)dst, C, MN, (int)ksplit);
     ctx->launches++;
   }
   TNCB_CUDA(cudaGetLastError());
@@ -501,6 +547,7 @@ __device__ __forceinline__ long long decomp_c(long long idx, const CompactLegs& 
   return off;
 }
 
+template <typename T>
 __global__ void __launch_bounds__(K0_THREADS)
 k0_batch_kernel(const K0BatchItem* __restrict__ items, const int* __restrict__ block_start, int n_items, char* __restrict__ ws) {
   int lo = 0, hi = n_items;
@@ -516,8 +563,8 @@ k0_batch_kernel(const K0BatchItem* __restrict__ items, const int* __restrict__ b
   const bool valid = o < MN;
   long long n = 0, m = 0;
   if (valid) { n = o / it.M; m = o - n * it.M; }
-  const double2* A = reinterpret_cast<const double2*>(ws + it.offA) + decomp_c(m, it.m);
-  const double2* B = reinterpret_cast<const double2*>(ws + it.offB) + decomp_c(n, it.n);
+  const T* A = reinterpret_cast<const T*>(ws + it.offA) + decomp_c(m, it.m);
+  const T* B = reinterpret_cast<const T*>(ws + it.offB) + decomp_c(n, it.n);
   double cr = 0.0, ci = 0.0;
   if (valid) {
     for (long long i = lane_g; i < it.K; i += G) {
@@ -528,8 +575,8 @@ k0_batch_kernel(const K0BatchItem* __restrict__ items, const int* __restrict__ b
         idx = q;
       }
       if (it.k.n > 0) { oa += idx * it.k.sa[0]; ob += idx * it.k.sb[0]; }
-      const double2 a = A[oa];
-      const double2 b = B[ob];
+      const double2 a = widen(A[oa]);
+      const double2 b = widen(B[ob]);
       cr = fma(b.x, a.x, cr); cr = fma(-b.y, a.y, cr);
       ci = fma(b.x, a.y, ci); ci = fma(b.y, a.x, ci);
     }
@@ -539,7 +586,7 @@ k0_batch_kernel(const K0BatchItem* __restrict__ items, const int* __restrict__ b
       cr += __shfl_xor_sync(0xffffffffu, cr, d);
       ci += __shfl_xor_sync(0xffffffffu, ci, d);
     }
-  if (valid && lane_g == 0) reinterpret_cast<double2*>(ws + it.offC)[o] = make_double2(cr, ci);
+  if (valid && lane_g == 0) st_round(reinterpret_cast<T*>(ws + it.offC) + o, cr, ci);
 }
 
 static bool compact_ok(const LegList& L) { return L.n <= kBatchGroups; }
@@ -566,19 +613,21 @@ int k0_batch_fill(int sm_count, const PairPlan& P, K0BatchItem* it) {
   return (int)((P.M * P.N + per_block - 1) / per_block);
 }
 
-int launch_k0_batch(tncb_ctx* ctx, const K0BatchItem* d_items, const int* d_block_start, int n_items, int total_blocks, char* ws) {
+int launch_k0_batch(tncb_ctx* ctx, const K0BatchItem* d_items, const int* d_block_start, int n_items, int total_blocks, char* ws,
+                    int dtype) {
   if (n_items <= 0 || total_blocks <= 0) return TNCB_OK;
-  k0_batch_kernel<<<(unsigned)total_blocks, K0_THREADS, 0, ctx->stream>>>(d_items, d_block_start, n_items, ws);
+  if (dtype == TNCB_C64) k0_batch_kernel<float2><<<(unsigned)total_blocks, K0_THREADS, 0, ctx->stream>>>(d_items, d_block_start, n_items, ws);
+  else k0_batch_kernel<double2><<<(unsigned)total_blocks, K0_THREADS, 0, ctx->stream>>>(d_items, d_block_start, n_items, ws);
   ctx->launches++;
   ctx->engine_count[0] += (uint64_t)n_items;
   TNCB_CUDA(cudaGetLastError());
   return TNCB_OK;
 }
 
-template <int BN, int BM, int WN, int WM, int ST, bool BKF, bool AKF, int MINB = 1>
+template <typename T, int BN, int BM, int WN, int WM, int ST, bool BKF, bool AKF, int MINB = 1>
 static int launch_k1_cfg(tncb_ctx* ctx, const K1Args& a) {
-  auto kern = k1_kernel<BN, BM, WN, WM, ST, BKF, AKF, MINB>;
-  const size_t smem = (size_t)ST * (BN * K1_BK + K1_BK * BM) * sizeof(double2);
+  auto kern = k1_kernel<BN, BM, WN, WM, ST, BKF, AKF, MINB, T>;
+  const size_t smem = (size_t)ST * (BN * K1_BK + K1_BK * BM) * sizeof(T);
   TNCB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const long long tiles = (long long)a.tiles_m * a.tiles_n * a.ksplit;
   if (tiles > 0x7fffffffLL) return fail(TNCB_ERR_UNSUPPORTED, "K1 grid too large");
@@ -590,7 +639,7 @@ static int launch_k1_cfg(tncb_ctx* ctx, const K1Args& a) {
   return TNCB_OK;
 }
 
-template <int BN, int BM, int WN, int WM, int ST, int MINB = 1>
+template <typename T, int BN, int BM, int WN, int WM, int ST, int MINB = 1>
 static int launch_k1_modes(tncb_ctx* ctx, K1Args& a, bool bkf, bool akf, bool allow_split) {
   a.tiles_m = (int)((a.M + BM - 1) / BM);
   a.tiles_n = (int)((a.N + BN - 1) / BN);
@@ -599,7 +648,7 @@ static int launch_k1_modes(tncb_ctx* ctx, K1Args& a, bool bkf, bool akf, bool al
   // fixed order afterwards (deterministic, no atomics).
   const long long tiles = (long long)a.tiles_m * a.tiles_n;
   const int nk_total = (int)((a.K + K1_BK - 1) / K1_BK);
-  double2* final_c = a.C;
+  T* final_c = static_cast<T*>(a.C);
   a.ksplit = 1; a.chunks_per_split = nk_total;
   const long long want_ctas = 2LL * ctx->sm_count;
   if (allow_split && tiles < want_ctas && nk_total >= 16) {
@@ -615,10 +664,10 @@ static int launch_k1_modes(tncb_ctx* ctx, K1Args& a, bool bkf, bool akf, bool al
     }
   }
   int rc;
-  if (bkf && akf) rc = launch_k1_cfg<BN, BM, WN, WM, ST, true, true, MINB>(ctx, a);
-  else if (bkf && !akf) rc = launch_k1_cfg<BN, BM, WN, WM, ST, true, false, MINB>(ctx, a);
-  else if (!bkf && akf) rc = launch_k1_cfg<BN, BM, WN, WM, ST, false, true, MINB>(ctx, a);
-  else rc = launch_k1_cfg<BN, BM, WN, WM, ST, false, false, MINB>(ctx, a);
+  if (bkf && akf) rc = launch_k1_cfg<T, BN, BM, WN, WM, ST, true, true, MINB>(ctx, a);
+  else if (bkf && !akf) rc = launch_k1_cfg<T, BN, BM, WN, WM, ST, true, false, MINB>(ctx, a);
+  else if (!bkf && akf) rc = launch_k1_cfg<T, BN, BM, WN, WM, ST, false, true, MINB>(ctx, a);
+  else rc = launch_k1_cfg<T, BN, BM, WN, WM, ST, false, false, MINB>(ctx, a);
   if (rc) return rc;
   ctx->engine_count[a.ksplit > 1 ? 3 : 2]++;
   if (a.ksplit > 1) {
@@ -630,7 +679,9 @@ static int launch_k1_modes(tncb_ctx* ctx, K1Args& a, bool bkf, bool akf, bool al
   return TNCB_OK;
 }
 
-static int launch_k1(tncb_ctx* ctx, const PairPlan& P, const double2* A, const double2* B, double2* C) {
+template <typename T>
+static int launch_k1(tncb_ctx* ctx, const PairPlan& P, const T* A, const T* B, T* C) {
+  constexpr int dtype = sizeof(T) == sizeof(double2) ? TNCB_C128 : TNCB_C64;
   const size_t tab_elems = (size_t)(P.M + P.N + 2 * P.K);
   int rc = ensure_tab(ctx, tab_elems);
   if (rc) return rc;
@@ -654,18 +705,18 @@ static int launch_k1(tncb_ctx* ctx, const PairPlan& P, const double2* A, const d
   // (CRT) emulation, crt.cu; the 7-bit digit-slicing engine of round 1 (ozaki.cu) stays selectable for A/B.
   if (ctx->oz_slices > 0 && P.M >= 128 && P.N >= 128) {
     static const bool force = std::getenv("TNCB_FORCE_TCGEN05") != nullptr;  // tuning aid: skip the size heuristic
-    if (ctx->oz_engine == 0) {
+    if (ctx->oz_engine == 0 || dtype == TNCB_C64) {   // (the digit-slicing engine has no complex64 path)
       const double mnk = (double)P.M * (double)P.N * (double)P.K;
       if (force || (P.K >= ctx->crt_min_k && mnk >= ctx->crt_min_mnk)) {
-        int rc = launch_k1_crt(ctx, P, A, B, C, a.offAm, a.offBn, a.offAk, a.offBk);
+        int rc = launch_k1_crt(ctx, P, A, B, C, a.offAm, a.offBn, a.offAk, a.offBk, dtype);
         if (rc != TNCB_ERR_OOM && rc != TNCB_ERR_UNSUPPORTED) return rc;   // no room for the residue planes: DMMA engine
       }
-    } else if (P.M >= 256 && P.N >= 256 && P.K >= 256) {
+    } else if (dtype == TNCB_C128 && P.M >= 256 && P.N >= 256 && P.K >= 256) {
       const long long tiles = ((P.M + 127) / 128) * ((P.N + 127) / 128);
       // crossover measured on B200 (profiles/r01_engine_sweep.txt): short K is dominated by the S
       // FP64 read-modify-write flushes per tile, few tiles leave SMs idle (1 CTA per 128x128 tile)
       if (force || (tiles >= ctx->oz_min_tiles && P.K >= ctx->oz_min_k) || (tiles >= 1024 && P.K >= 1024)) {
-        int rc = launch_k1_ozaki(ctx, P, A, B, C, ctx->oz_slices, a.offAm, a.offBn, a.offAk, a.offBk);
+        int rc = launch_k1_ozaki(ctx, P, (const double2*)A, (const double2*)B, (double2*)C, ctx->oz_slices, a.offAm, a.offBn, a.offAk, a.offBk);
         if (rc == TNCB_OK) ctx->engine_count[4]++;
         if (rc != TNCB_ERR_OOM) return rc;   // no room for the digit planes: fall through to the DMMA engine
       }
@@ -676,10 +727,10 @@ static int launch_k1(tncb_ctx* ctx, const PairPlan& P, const double2* A, const d
   // hide each other's per-chunk barrier/gather bubbles); 128x64 with 3-4 stages and 1 CTA/SM
   // stays at 75-81 %.  Skinny outputs use a 32-wide tile on the narrow side.
   static const int variant = std::getenv("TNCB_K1_VARIANT") ? atoi(std::getenv("TNCB_K1_VARIANT")) : 0;
-  if (variant == 1) return launch_k1_modes<128, 64, 4, 2, 4, 1>(ctx, a, P.b_kfast, P.a_kfast, true);
-  if (P.N <= 32 && P.M > 32) return launch_k1_modes<32, 64, 1, 2, 2, 2>(ctx, a, P.b_kfast, P.a_kfast, true);
-  if (P.M <= 32 && P.N > 32) return launch_k1_modes<64, 32, 2, 1, 2, 2>(ctx, a, P.b_kfast, P.a_kfast, true);
-  return launch_k1_modes<64, 64, 2, 2, 2, 2>(ctx, a, P.b_kfast, P.a_kfast, true);
+  if (variant == 1) return launch_k1_modes<T, 128, 64, 4, 2, 4, 1>(ctx, a, P.b_kfast, P.a_kfast, true);
+  if (P.N <= 32 && P.M > 32) return launch_k1_modes<T, 32, 64, 1, 2, 2, 2>(ctx, a, P.b_kfast, P.a_kfast, true);
+  if (P.M <= 32 && P.N > 32) return launch_k1_modes<T, 64, 32, 2, 1, 2, 2>(ctx, a, P.b_kfast, P.a_kfast, true);
+  return launch_k1_modes<T, 64, 64, 2, 2, 2, 2>(ctx, a, P.b_kfast, P.a_kfast, true);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -712,9 +763,9 @@ __device__ __forceinline__ long long decomp_shift(long long idx, const LegList& 
   return off;
 }
 
-template <int NS>
+template <int NS, typename T>
 __global__ void __launch_bounds__(256)
-k2_kernel(const double2* __restrict__ Big, const double2* __restrict__ Sml, double2* __restrict__ C,
+k2_kernel(const T* __restrict__ Big, const T* __restrict__ Sml, T* __restrict__ C,
           const __grid_constant__ K2Args p) {
   __shared__ double2 s_s[16 * 64];     // S[s][k], s < NS, k < K <= 64 ... NS*K <= 256 guaranteed by the planner
   __shared__ long long s_kbig[64];
@@ -730,7 +781,7 @@ k2_kernel(const double2* __restrict__ Big, const double2* __restrict__ Sml, doub
     if (sidx < p.SMALL) {
       long long ob, os;
       decomp_ab(k, p.k, ob, os);
-      v = __ldg(Sml + decomp_a(sidx, p.sml) + os);
+      v = ldg_wide(Sml + decomp_a(sidx, p.sml) + os);
     }
     s_s[i] = v;
   }
@@ -741,7 +792,7 @@ k2_kernel(const double2* __restrict__ Big, const double2* __restrict__ Sml, doub
 #pragma unroll
     for (int sI = 0; sI < NS; sI++) { ar[sI] = 0.0; ai[sI] = 0.0; }
     for (int k = 0; k < K; k++) {
-      const double2 v = __ldg(Big + off + s_kbig[k]);
+      const double2 v = ldg_wide(Big + off + s_kbig[k]);
 #pragma unroll
       for (int sI = 0; sI < NS; sI++) {
         const double2 w = s_s[sI * K + k];   // broadcast
@@ -752,17 +803,18 @@ k2_kernel(const double2* __restrict__ Big, const double2* __restrict__ Sml, doub
     if (p.big_is_a) {
 #pragma unroll
       for (int sI = 0; sI < NS; sI++)
-        if (sI < p.SMALL) C[(long long)sI * p.M + x] = make_double2(ar[sI], ai[sI]);
+        if (sI < p.SMALL) st_round(C + (long long)sI * p.M + x, ar[sI], ai[sI]);
     } else {
-      double2* dst = C + x * p.M;
+      T* dst = C + x * p.M;
 #pragma unroll
       for (int sI = 0; sI < NS; sI++)
-        if (sI < p.SMALL) dst[sI] = make_double2(ar[sI], ai[sI]);
+        if (sI < p.SMALL) st_round(dst + sI, ar[sI], ai[sI]);
     }
   }
 }
 
-static int launch_k2(tncb_ctx* ctx, const PairPlan& P, const double2* A, const double2* B, double2* C) {
+template <typename T>
+static int launch_k2(tncb_ctx* ctx, const PairPlan& P, const T* A, const T* B, T* C) {
   K2Args a;
   const bool big_a = P.k2_big_is_a;
   a.big = big_a ? P.m : P.n;
@@ -775,16 +827,16 @@ static int launch_k2(tncb_ctx* ctx, const PairPlan& P, const double2* A, const d
     const long long d = a.big.dim[g];
     if (d & (d - 1)) { a.pow2 = 0; a.shift[g] = 0; } else { int sh = 0; while ((1LL << sh) < d) sh++; a.shift[g] = sh; }
   }
-  const double2* Big = big_a ? A : B;
-  const double2* Sml = big_a ? B : A;
+  const T* Big = big_a ? A : B;
+  const T* Sml = big_a ? B : A;
   const int blocks = (int)std::min<long long>((a.BIG + 255) / 256, (long long)ctx->sm_count * 32);
   int ns = 1; while (ns < a.SMALL) ns *= 2;
   switch (ns) {
-    case 1: k2_kernel<1><<<blocks, 256, 0, ctx->stream>>>(Big, Sml, C, a); break;
-    case 2: k2_kernel<2><<<blocks, 256, 0, ctx->stream>>>(Big, Sml, C, a); break;
-    case 4: k2_kernel<4><<<blocks, 256, 0, ctx->stream>>>(Big, Sml, C, a); break;
-    case 8: k2_kernel<8><<<blocks, 256, 0, ctx->stream>>>(Big, Sml, C, a); break;
-    default: k2_kernel<16><<<blocks, 256, 0, ctx->stream>>>(Big, Sml, C, a); break;
+    case 1: k2_kernel<1, T><<<blocks, 256, 0, ctx->stream>>>(Big, Sml, C, a); break;
+    case 2: k2_kernel<2, T><<<blocks, 256, 0, ctx->stream>>>(Big, Sml, C, a); break;
+    case 4: k2_kernel<4, T><<<blocks, 256, 0, ctx->stream>>>(Big, Sml, C, a); break;
+    case 8: k2_kernel<8, T><<<blocks, 256, 0, ctx->stream>>>(Big, Sml, C, a); break;
+    default: k2_kernel<16, T><<<blocks, 256, 0, ctx->stream>>>(Big, Sml, C, a); break;
   }
   ctx->launches++;
   ctx->engine_count[5]++;
@@ -792,12 +844,18 @@ static int launch_k2(tncb_ctx* ctx, const PairPlan& P, const double2* A, const d
   return TNCB_OK;
 }
 
-int launch_pair(tncb_ctx* ctx, const PairPlan& P, const double2* A, const double2* B, double2* C) {
-  if (P.M * P.N == 0) return TNCB_OK;
-  NvtxPairRange nvtx_range(P);
+template <typename T>
+static int launch_pair_t(tncb_ctx* ctx, const PairPlan& P, const T* A, const T* B, T* C) {
   if (P.kernel_class == 2) return launch_k2(ctx, P, A, B, C);
   if (P.kernel_class == 1) return launch_k1(ctx, P, A, B, C);
   return launch_k0(ctx, P, A, B, C);
+}
+
+int launch_pair(tncb_ctx* ctx, const PairPlan& P, const void* A, const void* B, void* C, int dtype) {
+  if (P.M * P.N == 0) return TNCB_OK;
+  NvtxPairRange nvtx_range(P);
+  if (dtype == TNCB_C64) return launch_pair_t(ctx, P, (const float2*)A, (const float2*)B, (float2*)C);
+  return launch_pair_t(ctx, P, (const double2*)A, (const double2*)B, (double2*)C);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -851,11 +909,12 @@ __global__ void k3_tables_kernel(const __grid_constant__ K3Args p, long long* __
   }
 }
 
+template <typename T>
 __global__ void __launch_bounds__(256)
-k3_transpose_kernel(const double2* __restrict__ in, double2* __restrict__ out, const __grid_constant__ K3Args p,
+k3_transpose_kernel(const T* __restrict__ in, T* __restrict__ out, const __grid_constant__ K3Args p,
                     const long long* __restrict__ tab) {
   extern __shared__ __align__(16) unsigned char k3_smem_raw[];
-  double2* tile = reinterpret_cast<double2*>(k3_smem_raw);
+  T* tile = reinterpret_cast<T*>(k3_smem_raw);
   // block index -> base offsets; room left in every partially tiled group
   long long b = blockIdx.x, base_in = 0, base_out = 0;
   int room[K3_MAXT];                                  // valid indices of tile group g in this tile: i < room[g]
@@ -894,8 +953,9 @@ k3_transpose_kernel(const double2* __restrict__ in, double2* __restrict__ out, c
   }
 }
 
-int launch_permute(tncb_ctx* ctx, const double2* in, double2* out, int rank,
-                   const uint64_t* in_dims, const int* perm) {
+template <typename T>
+static int launch_permute_t(tncb_ctx* ctx, const T* in, T* out, int rank,
+                            const uint64_t* in_dims, const int* perm) {
   std::vector<long long> istr(rank);
   long long s = 1, total = 1;
   for (int i = rank - 1; i >= 0; i--) { istr[i] = s; s *= (long long)in_dims[i]; }
@@ -915,7 +975,7 @@ int launch_permute(tncb_ctx* ctx, const double2* in, double2* out, int rank,
   static const bool no_tiled = std::getenv("TNCB_NO_K3") != nullptr;
   if (n <= 1 || no_tiled || total < 4096) {   // identity / tiny: the plain gather kernel (already coalesced or negligible)
     const int blocks = (int)std::min<long long>((total + 255) / 256, (long long)ctx->sm_count * 16);
-    permute_kernel<<<blocks, 256, 0, ctx->stream>>>(in, out, L, total);
+    permute_kernel<T><<<blocks, 256, 0, ctx->stream>>>(in, out, L, total);
     ctx->launches++;
     TNCB_CUDA(cudaGetLastError());
     return TNCB_OK;
@@ -972,7 +1032,7 @@ int launch_permute(tncb_ctx* ctx, const double2* in, double2* out, int rank,
   for (int k = 0; k < a.nt; k++) { const int g = tg[k]; a.ext[k] = ext[g]; a.dim[k] = L.dim[g]; a.sin[k] = L.sa[g]; a.sout[k] = ostr[g]; te *= ext[g]; }
   if (plain || te > K3_TILE || te < 64) {   // degenerate tilings: the plain gather kernel
     const int blocks = (int)std::min<long long>((total + 255) / 256, (long long)ctx->sm_count * 16);
-    permute_kernel<<<blocks, 256, 0, ctx->stream>>>(in, out, L, total);
+    permute_kernel<T><<<blocks, 256, 0, ctx->stream>>>(in, out, L, total);
     ctx->launches++;
     TNCB_CUDA(cudaGetLastError());
     return TNCB_OK;
@@ -992,40 +1052,49 @@ int launch_permute(tncb_ctx* ctx, const double2* in, double2* out, int rank,
   }
   for (int g = 0; g < n; g++) if (ext[g] == 1) { a.rcount[a.nr] = L.dim[g]; a.rin[a.nr] = L.sa[g]; a.rout[a.nr] = ostr[g]; a.rtile[a.nr] = -1; a.nr++; blocks *= L.dim[g]; }
   if (blocks > 0x7fffffffLL) return fail(TNCB_ERR_UNSUPPORTED, "permute grid too large");
-  const int smem = (int)((te + te / 32 + 1) * sizeof(double2));
-  static bool attr_done_dev[64] = {false};          // cudaFuncSetAttribute is per device
+  const int smem = (int)((te + te / 32 + 1) * sizeof(T));
+  static bool attr_done_dev[64] = {false};          // cudaFuncSetAttribute is per device (and per instantiation)
   bool& attr_done = attr_done_dev[ctx->device & 63];
-  if (!attr_done) { TNCB_CUDA(cudaFuncSetAttribute(k3_transpose_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (K3_TILE + K3_TILE / 32 + 1) * (int)sizeof(double2))); attr_done = true; }
+  if (!attr_done) { TNCB_CUDA(cudaFuncSetAttribute(k3_transpose_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (K3_TILE + K3_TILE / 32 + 1) * (int)sizeof(T))); attr_done = true; }
   int rc = ensure_tab(ctx, (size_t)(5 * te));
   if (rc) return rc;
   ctx->tab_valid = false;                       // the K1 offset tables living in the same buffer are gone
   k3_tables_kernel<<<(unsigned)((te + 255) / 256), 256, 0, ctx->stream>>>(a, ctx->tab);
-  k3_transpose_kernel<<<(unsigned)blocks, 256, smem, ctx->stream>>>(in, out, a, ctx->tab);
+  k3_transpose_kernel<T><<<(unsigned)blocks, 256, smem, ctx->stream>>>(in, out, a, ctx->tab);
   ctx->launches += 2;
   TNCB_CUDA(cudaGetLastError());
   return TNCB_OK;
 }
 
-__global__ void add_kernel(double2* __restrict__ dst, const double2* __restrict__ src, long long total) {
+int launch_permute(tncb_ctx* ctx, const void* in, void* out, int rank, const uint64_t* in_dims, const int* perm, int dtype) {
+  if (dtype == TNCB_C64) return launch_permute_t(ctx, (const float2*)in, (float2*)out, rank, in_dims, perm);
+  return launch_permute_t(ctx, (const double2*)in, (double2*)out, rank, in_dims, perm);
+}
+
+// complex64: the sum of two complex64 values, rounded once (numpy's complex64 addition)
+template <typename T>
+__global__ void add_kernel(T* __restrict__ dst, const T* __restrict__ src, long long total) {
   for (long long o = (long long)blockIdx.x * blockDim.x + threadIdx.x; o < total; o += (long long)gridDim.x * blockDim.x) {
-    double2 d = dst[o]; const double2 v = src[o];
+    T d = dst[o]; const T v = src[o];
     d.x += v.x; d.y += v.y; dst[o] = d;
   }
 }
 
-int launch_add(tncb_ctx* ctx, double2* dst, const double2* src, uint64_t elems) {
+int launch_add(tncb_ctx* ctx, void* dst, const void* src, uint64_t elems, int dtype) {
   if (elems == 0) return TNCB_OK;
   const int blocks = (int)std::min<long long>(((long long)elems + 255) / 256, (long long)ctx->sm_count * 16);
-  add_kernel<<<blocks, 256, 0, ctx->stream>>>(dst, src, (long long)elems);
+  if (dtype == TNCB_C64) add_kernel<float2><<<blocks, 256, 0, ctx->stream>>>((float2*)dst, (const float2*)src, (long long)elems);
+  else add_kernel<double2><<<blocks, 256, 0, ctx->stream>>>((double2*)dst, (const double2*)src, (long long)elems);
   ctx->launches++;
   TNCB_CUDA(cudaGetLastError());
   return TNCB_OK;
 }
 
-int launch_conj(tncb_ctx* ctx, double2* data, uint64_t elems) {
+int launch_conj(tncb_ctx* ctx, void* data, uint64_t elems, int dtype) {
   if (elems == 0) return TNCB_OK;
   const int blocks = (int)std::min<long long>(((long long)elems + 255) / 256, (long long)ctx->sm_count * 16);
-  conj_kernel<<<blocks, 256, 0, ctx->stream>>>(data, (long long)elems);
+  if (dtype == TNCB_C64) conj_kernel<float2><<<blocks, 256, 0, ctx->stream>>>((float2*)data, (long long)elems);
+  else conj_kernel<double2><<<blocks, 256, 0, ctx->stream>>>((double2*)data, (long long)elems);
   ctx->launches++;
   TNCB_CUDA(cudaGetLastError());
   return TNCB_OK;

@@ -34,8 +34,10 @@ struct Schedule {
   size_t leaf_block_elems = 0;
   std::vector<Step> steps;
   int result_slot = -1;
-  double flops = 0, bytes = 0;
+  double flops = 0, bytes = 0;      // bytes at 16 B per element (PairPlan::bytes); scaled by esz() / 16 where reported
   size_t n_leaves_total = 0;
+  int dtype = TNCB_C128;            // element type of every device tensor of the run (host payloads stay complex128)
+  size_t esz() const { return dtype_size(dtype); }
 };
 
 static const tncb_path* find_nested(const tncb_path* path, size_t idx) {
@@ -71,6 +73,7 @@ static int add_leaf(const tncb_tn* leaf, Schedule& S, size_t leaf_idx, int* slot
     if (!leaf->host_re_im) return fail(TNCB_ERR_INVALID, "matrix leaf without host data");
   } else if (leaf->kind == TNCB_DATA_DEVICE) {
     if (!leaf->device) return fail(TNCB_ERR_INVALID, "device leaf without a tensor handle");
+    if (leaf->device->dtype != S.dtype) return fail(TNCB_ERR_INVALID, "device leaf: dtype differs from the network's");
     if (leaf->device->elems != m.elems) return fail(TNCB_ERR_SHAPE, "device leaf: element count mismatch");
   } else if (leaf->kind == TNCB_DATA_FILE) {
     if (!leaf->file_path) return fail(TNCB_ERR_INVALID, "file leaf without a path");
@@ -144,8 +147,10 @@ static int build(const tncb_tn* tn, const tncb_path* path, Schedule& S, size_t& 
   return TNCB_OK;
 }
 
-static int build_schedule(const tncb_tn* tn, const tncb_path* path, Schedule& S) {
+static int build_schedule(const tncb_tn* tn, const tncb_path* path, Schedule& S, int dtype = TNCB_C128) {
   if (!tn) return fail(TNCB_ERR_INVALID, "tn is null");
+  if (!dtype_size(dtype)) return fail(TNCB_ERR_INVALID, "dtype must be TNCB_C128 or TNCB_C64");
+  S.dtype = dtype;
   S.n_leaves_total = count_leaves(tn);
   S.leaf_offset.assign(S.n_leaves_total, 0);
   S.leaf_kind.assign(S.n_leaves_total, TNCB_DATA_UNCONTRACTED);
@@ -179,6 +184,7 @@ static int validate_leaves(const Schedule& S, const std::vector<const tncb_tn*>&
     if (lf->kind == TNCB_DATA_FILE && !lf->file_path) return fail(TNCB_ERR_INVALID, "file leaf " + std::to_string(li) + " without a path");
     if (lf->kind == TNCB_DATA_DEVICE) {
       if (!lf->device || !lf->device->ptr) return fail(TNCB_ERR_UNCONTRACTED, "device leaf " + std::to_string(li) + " without a tensor handle (already consumed?)");
+      if (lf->device->dtype != S.dtype) return fail(TNCB_ERR_INVALID, "device leaf " + std::to_string(li) + ": dtype differs from the plan's");
       if (lf->device->elems != m->elems) return fail(TNCB_ERR_SHAPE, "device leaf " + std::to_string(li) + ": element count mismatch");
     }
   }
@@ -190,17 +196,18 @@ static int validate_leaves(const Schedule& S, const std::vector<const tncb_tn*>&
   return TNCB_OK;
 }
 
-static int stage_leaves(const Schedule& S, const std::vector<const tncb_tn*>& leaves, std::complex<double>* stage);
+static int stage_leaves(const Schedule& S, const std::vector<const tncb_tn*>& leaves, void* stage);
 
 // `resident` != nullptr: the leaf block already sits on the device (tncb_plan_stage); `tn` may then be null.
 static int execute(tncb_ctx* ctx, const Schedule& S, const tncb_tn* tn, tncb_tensor** out, int* n_out, uint64_t* out_legs,
-                   const double2* resident = nullptr) {
+                   const void* resident = nullptr) {
+  const size_t esz = S.esz();
   TNCB_CUDA(cudaSetDevice(ctx->device));
   std::vector<const tncb_tn*> leaves;
   if (tn) collect_leaf_nodes(tn, leaves);
   if (!resident) { int vrc = validate_leaves(S, leaves); if (vrc) return vrc; }
   // ---- stage all host payloads, one H2D copy ----
-  const size_t block_bytes = resident ? 0 : S.leaf_block_elems * sizeof(double2);
+  const size_t block_bytes = resident ? 0 : S.leaf_block_elems * esz;
   void* leaf_block = nullptr;
   if (block_bytes) {
     if (ctx->stage_bytes < block_bytes) {
@@ -212,19 +219,19 @@ static int execute(tncb_ctx* ctx, const Schedule& S, const tncb_tn* tn, tncb_ten
       // the previous network's upload may still be reading the staging buffer
       TNCB_CUDA(cudaStreamSynchronize(ctx->stream));
     }
-    { int src = stage_leaves(S, leaves, (std::complex<double>*)ctx->stage_host); if (src) return src; }
+    { int src = stage_leaves(S, leaves, ctx->stage_host); if (src) return src; }
     int rc = ctx->arena.alloc(block_bytes, &leaf_block);
     if (rc) return rc;
     TNCB_CUDA(cudaMemcpyAsync(leaf_block, ctx->stage_host, block_bytes, cudaMemcpyHostToDevice, ctx->stream));
   }
   // ---- run the schedule ----
-  struct Live { double2* ptr = nullptr; size_t bytes = 0; tncb_tensor* handle = nullptr; };
+  struct Live { char* ptr = nullptr; size_t bytes = 0; tncb_tensor* handle = nullptr; };
   std::vector<Live> live(S.slots.size());
   for (size_t s = 0; s < S.slots.size(); s++) {
     const int li = S.slots[s].leaf_index;
     if (li < 0) continue;
-    if (S.leaf_kind[li] == TNCB_DATA_DEVICE) { live[s].ptr = leaves[li]->device->ptr; live[s].handle = leaves[li]->device; }
-    else live[s].ptr = (resident ? const_cast<double2*>(resident) : (double2*)leaf_block) + S.leaf_offset[li];
+    if (S.leaf_kind[li] == TNCB_DATA_DEVICE) { live[s].ptr = (char*)leaves[li]->device->ptr; live[s].handle = leaves[li]->device; }
+    else live[s].ptr = (resident ? (char*)const_cast<void*>(resident) : (char*)leaf_block) + S.leaf_offset[li] * esz;
   }
   int rc = TNCB_OK;
   std::vector<tncb_tensor*> consumed;
@@ -235,11 +242,11 @@ static int execute(tncb_ctx* ctx, const Schedule& S, const tncb_tn* tn, tncb_ten
   size_t step_no = 0;
   for (const Step& st : S.steps) {
     const SlotMeta& om = S.slots[st.out];
-    size_t bytes = std::max<size_t>(om.elems * sizeof(double2), 16);
+    size_t bytes = std::max<size_t>(om.elems * esz, 16);
     void* p = nullptr;
     if ((rc = ctx->arena.alloc(bytes, &p))) break;
-    live[st.out].ptr = (double2*)p; live[st.out].bytes = bytes;
-    if ((rc = launch_pair(ctx, st.plan, live[st.a].ptr, live[st.b].ptr, live[st.out].ptr))) break;
+    live[st.out].ptr = (char*)p; live[st.out].bytes = bytes;
+    if ((rc = launch_pair(ctx, st.plan, live[st.a].ptr, live[st.b].ptr, live[st.out].ptr, S.dtype))) break;
     for (int s : {st.a, st.b}) { // operands are consumed (mem::take, contraction.rs:61-62)
       // caller-owned device leaves are released only after the WHOLE schedule was enqueued (atomic consumption:
       // on any error every device input is still alive and owned by the caller, see tncb.h)
@@ -256,7 +263,7 @@ static int execute(tncb_ctx* ctx, const Schedule& S, const tncb_tn* tn, tncb_ten
       const PairPlan& P = S.steps[q].plan;
       fprintf(stderr, "TNCB_TRACE step %zu class K%d M %lld N %lld K %lld groups m%d n%d k%d akf %d bkf %d ms %.4f tflops %.2f gbs %.1f\n",
               q, P.kernel_class, P.M, P.N, P.K, P.m.n, P.n.n, P.k.n, (int)P.a_kfast, (int)P.b_kfast, ms,
-              P.flops() / (ms * 1e-3) * 1e-12, P.bytes() / (ms * 1e-3) * 1e-9);
+              P.flops() / (ms * 1e-3) * 1e-12, P.bytes() * (double)esz / 16.0 / (ms * 1e-3) * 1e-9);
     }
     for (auto& e : tev) cudaEventDestroy(e);
   }
@@ -265,19 +272,19 @@ static int execute(tncb_ctx* ctx, const Schedule& S, const tncb_tn* tn, tncb_ten
     const SlotMeta& rm = S.slots[S.result_slot];
     Live& rl = live[S.result_slot];
     result = new tncb_tensor();
-    result->rank = (int)rm.dims.size(); result->elems = rm.elems;
+    result->rank = (int)rm.dims.size(); result->elems = rm.elems; result->dtype = S.dtype;
     for (size_t i = 0; i < rm.dims.size(); i++) result->dims[i] = rm.dims[i];
     if (rl.bytes) { // produced by a pair: hand the arena block over
-      result->ptr = rl.ptr; result->bytes = rl.bytes; rl.bytes = 0;
+      result->ptr = (double2*)rl.ptr; result->bytes = rl.bytes; rl.bytes = 0;
     } else if (rl.handle) { // a device leaf that was never contracted: the result takes its storage over
       *result = *rl.handle; rl.handle->ptr = nullptr; rl.handle->bytes = 0; consumed.push_back(rl.handle); rl.handle = nullptr;
     } else { // an uploaded leaf that was never contracted: copy it out of the leaf block
-      result->bytes = std::max<size_t>(rm.elems * sizeof(double2), 16);
+      result->bytes = std::max<size_t>(rm.elems * esz, 16);
       void* p = nullptr;
       rc = ctx->arena.alloc(result->bytes, &p);
       if (!rc) {
         result->ptr = (double2*)p;
-        cudaMemcpyAsync(p, rl.ptr, rm.elems * sizeof(double2), cudaMemcpyDeviceToDevice, ctx->stream);
+        cudaMemcpyAsync(p, rl.ptr, rm.elems * esz, cudaMemcpyDeviceToDevice, ctx->stream);
       } else { delete result; result = nullptr; }
     }
   }
@@ -389,17 +396,18 @@ static void plan_static_layout(tncb_plan* P, int sm_count, size_t device_bytes) 
   size_t scratch = 0;
   for (const Step& st : S.steps) if (st.plan.kernel_class == 0) scratch = std::max(scratch, k0_partial_elems(sm_count, st.plan));
   OffsetAlloc A;
-  P->leaf_off = A.alloc(std::max<size_t>(S.leaf_block_elems * sizeof(double2), 16));
+  const size_t esz = S.esz();
+  P->leaf_off = A.alloc(std::max<size_t>(S.leaf_block_elems * esz, 16));
   P->scratch_elems = scratch;
-  P->scratch_off = scratch ? A.alloc(scratch * sizeof(double2)) : 0;
+  P->scratch_off = scratch ? A.alloc(scratch * sizeof(double2)) : 0;   // split-K partials are f64 for both dtypes
   P->slot_off.assign(S.slots.size(), 0);
   std::vector<size_t> sz(S.slots.size(), 0);
   for (size_t s2 = 0; s2 < S.slots.size(); s2++)
-    if (S.slots[s2].leaf_index >= 0) P->slot_off[s2] = P->leaf_off + S.leaf_offset[S.slots[s2].leaf_index] * sizeof(double2);
+    if (S.slots[s2].leaf_index >= 0) P->slot_off[s2] = P->leaf_off + S.leaf_offset[S.slots[s2].leaf_index] * esz;
   for (int l = 0; l < n_levels; l++) {
     for (int q = P->level_begin[l]; q < P->level_begin[l + 1]; q++) {
       const Step& st = S.steps[q];
-      sz[st.out] = std::max<size_t>(S.slots[st.out].elems * sizeof(double2), 16);
+      sz[st.out] = std::max<size_t>(S.slots[st.out].elems * esz, 16);
       P->slot_off[st.out] = A.alloc(sz[st.out]);
     }
     for (int q = P->level_begin[l]; q < P->level_begin[l + 1]; q++) {
@@ -435,19 +443,35 @@ static void plan_static_layout(tncb_plan* P, int sm_count, size_t device_bytes) 
   for (const Step& st : S.steps) if (st.plan.kernel_class == 1) { P->graphable = false; break; }   // K1/K1' use ctx-owned tables / arena scratch
 }
 
-static int stage_leaves(const Schedule& S, const std::vector<const tncb_tn*>& leaves, std::complex<double>* stage) {
+// Host payloads are complex128; a complex64 run narrows them (one rounding per part) as they go into the staging block.
+static int stage_leaves(const Schedule& S, const std::vector<const tncb_tn*>& leaves, void* stage_v) {
+  const bool c64 = S.dtype == TNCB_C64;
+  std::complex<double>* stage = (std::complex<double>*)stage_v;
+  std::vector<std::complex<double>> wide;   // complex64 runs: gate / file payloads before narrowing
   for (size_t li = 0; li < leaves.size(); li++) {
     const tncb_tn* lf = leaves[li];
     if (S.leaf_kind[li] != lf->kind) return fail(TNCB_ERR_INVALID, "network payload kinds do not match the plan");
+    if (lf->kind != TNCB_DATA_GATE && lf->kind != TNCB_DATA_MATRIX && lf->kind != TNCB_DATA_FILE) continue;
+    uint64_t e = 1; for (int i = 0; i < lf->rank; i++) e *= lf->dims[i];
+    const double* src = nullptr;
+    if (c64 && lf->kind != TNCB_DATA_MATRIX) wide.resize(std::max<uint64_t>(e, 16));
+    std::complex<double>* dst = c64 ? wide.data() : stage + S.leaf_offset[li];
     if (lf->kind == TNCB_DATA_GATE) {
-      int cnt = gate_matrix(lf->gate_name, lf->gate_angles, lf->n_gate_angles, lf->gate_adjoint != 0, stage + S.leaf_offset[li]);
+      int cnt = gate_matrix(lf->gate_name, lf->gate_angles, lf->n_gate_angles, lf->gate_adjoint != 0, dst);
       if (cnt < 0) return cnt;
+      e = (uint64_t)cnt;
+      src = (const double*)dst;
     } else if (lf->kind == TNCB_DATA_MATRIX) {
-      uint64_t e = 1; for (int i = 0; i < lf->rank; i++) e *= lf->dims[i];
-      std::memcpy(stage + S.leaf_offset[li], lf->host_re_im, e * sizeof(double2));
-    } else if (lf->kind == TNCB_DATA_FILE) {      // into_data for TensorData::File (tensordata.rs:43-49)
-      int rc = h5::load_file_leaf(lf->file_path, lf->file_adjoint != 0, lf->rank, lf->dims, (double*)(stage + S.leaf_offset[li]));
+      if (!c64) std::memcpy(stage + S.leaf_offset[li], lf->host_re_im, e * sizeof(double2));
+      src = lf->host_re_im;
+    } else {      // into_data for TensorData::File (tensordata.rs:43-49)
+      int rc = h5::load_file_leaf(lf->file_path, lf->file_adjoint != 0, lf->rank, lf->dims, (double*)dst);
       if (rc) return rc;
+      src = (const double*)dst;
+    }
+    if (c64) {
+      float* d = (float*)stage_v + 2 * S.leaf_offset[li];
+      for (uint64_t i = 0; i < 2 * e; i++) d[i] = (float)src[i];
     }
   }
   return TNCB_OK;
@@ -459,7 +483,7 @@ static int plan_device_state(tncb_ctx* ctx, tncb_plan* P) {
   if (!P->ctx) { P->ctx = ctx; ctx->plans.push_back(P); }
   int rc;
   if (!P->ws && (rc = ctx->arena.alloc(P->ws_bytes, &P->ws))) return rc;
-  const size_t block_bytes = std::max<size_t>(P->S.leaf_block_elems * sizeof(double2), 16);
+  const size_t block_bytes = std::max<size_t>(P->S.leaf_block_elems * P->S.esz(), 16);
   if (!P->stage) TNCB_CUDA(cudaMallocHost(&P->stage, block_bytes));
   if (!P->batch_dev && !P->items.empty()) {
     const size_t ib = P->items.size() * sizeof(K0BatchItem), bb = P->block_start.size() * sizeof(int);
@@ -486,12 +510,11 @@ static int enqueue_static(tncb_ctx* ctx, tncb_plan* P) {
     const int nb = P->level_batched[l];
     if (nb) {
       const int total_blocks = P->block_start[P->bs_first[l] + nb];
-      rc = launch_k0_batch(ctx, d_items + P->item_first[l], d_bs + P->bs_first[l], nb, total_blocks, ws);
+      rc = launch_k0_batch(ctx, d_items + P->item_first[l], d_bs + P->bs_first[l], nb, total_blocks, ws, S.dtype);
     }
     for (int q = P->level_begin[l] + nb; q < P->level_begin[l + 1] && !rc; q++) {
       const Step& st = S.steps[q];
-      rc = launch_pair(ctx, st.plan, (const double2*)(ws + P->slot_off[st.a]), (const double2*)(ws + P->slot_off[st.b]),
-                       (double2*)(ws + P->slot_off[st.out]));
+      rc = launch_pair(ctx, st.plan, ws + P->slot_off[st.a], ws + P->slot_off[st.b], ws + P->slot_off[st.out], S.dtype);
     }
   }
   ctx->partial_override = nullptr; ctx->partial_override_elems = 0;
@@ -509,14 +532,14 @@ static int execute_static(tncb_ctx* ctx, tncb_plan* P, const tncb_tn* tn, tncb_t
     if ((rc = validate_leaves(S, leaves))) return rc;
   } else if (!P->leaves_resident) return fail(TNCB_ERR_INVALID, "tncb_plan_stage has not been called on this plan");
   if ((rc = plan_device_state(ctx, P))) return rc;
-  const size_t block_bytes = std::max<size_t>(S.leaf_block_elems * sizeof(double2), 16);
+  const size_t block_bytes = std::max<size_t>(S.leaf_block_elems * S.esz(), 16);
   char* ws = (char*)P->ws;
   const int which = tn ? 0 : 1;
   if (tn) {
     // an earlier upload may still read the staging buffer (it waits behind the previous network's kernels on the stream)
     if (P->exec[0] || P->leaves_resident) TNCB_CUDA(cudaStreamSynchronize(ctx->stream));
     else if (P->stage_busy) TNCB_CUDA(cudaEventSynchronize(P->stage_ev));
-    if ((rc = stage_leaves(S, leaves, (std::complex<double>*)P->stage))) return rc;
+    if ((rc = stage_leaves(S, leaves, P->stage))) return rc;
     P->leaves_resident = false;     // the workspace copy is about to be overwritten with this call's payloads
   }
   if (P->graphable) {
@@ -555,8 +578,8 @@ static int execute_static(tncb_ctx* ctx, tncb_plan* P, const tncb_tn* tn, tncb_t
   tncb_tensor* result = nullptr;
   if (S.result_slot >= 0) {
     const SlotMeta& rm = S.slots[S.result_slot];
-    if ((rc = tensor_new(ctx, (int)rm.dims.size(), rm.dims.data(), &result))) return rc;
-    TNCB_CUDA(cudaMemcpyAsync(result->ptr, ws + P->slot_off[S.result_slot], rm.elems * sizeof(double2), cudaMemcpyDeviceToDevice, ctx->stream));
+    if ((rc = tensor_new(ctx, (int)rm.dims.size(), rm.dims.data(), &result, S.dtype))) return rc;
+    TNCB_CUDA(cudaMemcpyAsync(result->ptr, ws + P->slot_off[S.result_slot], rm.elems * S.esz(), cudaMemcpyDeviceToDevice, ctx->stream));
   }
   if (out) *out = result; else if (result) tncb_tensor_free(ctx, result);
   if (n_out) *n_out = S.result_slot >= 0 ? (int)S.slots[S.result_slot].legs.size() : 0;
@@ -592,13 +615,20 @@ static void key_path(const tncb_path* p, std::vector<uint64_t>& k) {
 
 int tncb_contract_tensor_network(tncb_ctx* ctx, const tncb_tn* tn, const tncb_path* path,
                                  tncb_tensor** out, int* n_out, uint64_t* out_legs) {
+  return tncb_contract_tensor_network_dt(ctx, tn, path, TNCB_C128, out, n_out, out_legs);
+}
+
+int tncb_contract_tensor_network_dt(tncb_ctx* ctx, const tncb_tn* tn, const tncb_path* path, int dtype,
+                                    tncb_tensor** out, int* n_out, uint64_t* out_legs) {
   if (!ctx || !tn) return tncb::fail(TNCB_ERR_INVALID, "null argument");
+  if (!tncb::dtype_size(dtype)) return tncb::fail(TNCB_ERR_INVALID, "dtype must be TNCB_C128 or TNCB_C64");
   // Repeated contractions of the same circuit (other bitstrings, angles, or simply again) hit a small per-context cache
   // of compiled plans: no schedule construction, static layout, batched tiny pairs.  TNCB_PLAN_CACHE=0 disables it.
   static const bool cache_on = !(std::getenv("TNCB_PLAN_CACHE") && atoi(std::getenv("TNCB_PLAN_CACHE")) == 0) && std::getenv("TNCB_TRACE") == nullptr;
   if (cache_on) {
     std::vector<uint64_t> key;
     bool cacheable = true;
+    key.push_back(0x7b00000000000000ull | (uint64_t)dtype);
     key_tn(tn, key, &cacheable);
     key_path(path, key);
     if (cacheable) {
@@ -618,7 +648,7 @@ int tncb_contract_tensor_network(tncb_ctx* ctx, const tncb_tn* tn, const tncb_pa
       static thread_local std::vector<uint64_t> last_miss;
       if (last_miss == key) {
         tncb_plan* pl = nullptr;
-        if (tncb_plan_create(ctx, tn, path, &pl) == TNCB_OK && pl->is_static) {
+        if (tncb_plan_create_dt(ctx, tn, path, dtype, &pl) == TNCB_OK && pl->is_static) {
           size_t total = 0, free_b = 0, total_b = 0;
           for (auto& c : cache) total += c.plan->ws_bytes;
           cudaMemGetInfo(&free_b, &total_b);
@@ -637,16 +667,19 @@ int tncb_contract_tensor_network(tncb_ctx* ctx, const tncb_tn* tn, const tncb_pa
     }
   }
   tncb::Schedule S;
-  int rc = tncb::build_schedule(tn, path, S);
+  int rc = tncb::build_schedule(tn, path, S, dtype);
   if (rc) return rc;
   return tncb::execute(ctx, S, tn, out, n_out, out_legs);
 }
 
 int tncb_plan_create(tncb_ctx* ctx, const tncb_tn* tn, const tncb_path* path, tncb_plan** out) {
-  (void)ctx;
+  return tncb_plan_create_dt(ctx, tn, path, TNCB_C128, out);
+}
+
+int tncb_plan_create_dt(tncb_ctx* ctx, const tncb_tn* tn, const tncb_path* path, int dtype, tncb_plan** out) {
   if (!tn || !out) return tncb::fail(TNCB_ERR_INVALID, "null argument");
   tncb_plan* p = new tncb_plan();
-  int rc = tncb::build_schedule(tn, path, p->S);
+  int rc = tncb::build_schedule(tn, path, p->S, dtype);
   if (rc) { delete p; return rc; }
   size_t dev_free = 0, dev_total = 0;
   if (ctx) { cudaSetDevice(ctx->device); if (cudaMemGetInfo(&dev_free, &dev_total) != cudaSuccess) { dev_total = 0; cudaGetLastError(); } }
@@ -679,15 +712,15 @@ int tncb_plan_stage(tncb_ctx* ctx, tncb_plan* plan, const tncb_tn* tn) {
   tncb::collect_leaf_nodes(tn, leaves);
   int rc = tncb::validate_leaves(S, leaves);
   if (rc) return rc;
-  const size_t bytes = std::max<size_t>(S.leaf_block_elems * sizeof(double2), 16);
-  std::vector<std::complex<double>> host(std::max<size_t>(S.leaf_block_elems, 1));
+  const size_t bytes = std::max<size_t>(S.leaf_block_elems * S.esz(), 16);
+  std::vector<std::complex<double>> host(std::max<size_t>(S.leaf_block_elems, 1));   // (complex64 plans use the first half)
   if (plan->is_static && (rc = tncb::plan_device_state(ctx, plan))) {
     if (rc != TNCB_ERR_OOM || plan->ws) return rc;
     plan->is_static = false;    // the static workspace does not fit: resident leaf block + pair-by-pair executor
   }
   if (plan->is_static) {      // the leaf block lives inside the plan workspace
     TNCB_CUDA(cudaStreamSynchronize(ctx->stream));
-    if ((rc = tncb::stage_leaves(S, leaves, (std::complex<double>*)plan->stage))) return rc;
+    if ((rc = tncb::stage_leaves(S, leaves, plan->stage))) return rc;
     TNCB_CUDA(cudaMemcpyAsync((char*)plan->ws + plan->leaf_off, plan->stage, bytes, cudaMemcpyHostToDevice, ctx->stream));
     TNCB_CUDA(cudaStreamSynchronize(ctx->stream));
     plan->leaves_resident = true;
@@ -699,7 +732,7 @@ int tncb_plan_stage(tncb_ctx* ctx, tncb_plan* plan, const tncb_tn* tn) {
     if ((rc = ctx->arena.alloc(bytes, &plan->resident))) return rc;
     plan->resident_bytes = bytes;
   }
-  TNCB_CUDA(cudaMemcpyAsync(plan->resident, host.data(), S.leaf_block_elems * sizeof(double2), cudaMemcpyHostToDevice, ctx->stream));
+  TNCB_CUDA(cudaMemcpyAsync(plan->resident, host.data(), S.leaf_block_elems * S.esz(), cudaMemcpyHostToDevice, ctx->stream));
   TNCB_CUDA(cudaStreamSynchronize(ctx->stream));   // `host` dies with this frame
   return TNCB_OK;
 }
@@ -709,10 +742,10 @@ int tncb_plan_run(tncb_ctx* ctx, tncb_plan* plan, tncb_tensor** out, int* n_out,
   static const bool trace = std::getenv("TNCB_TRACE") != nullptr;
   if (plan->is_static && plan->leaves_resident && plan->ctx == ctx) {
     if (!trace) return tncb::execute_static(ctx, plan, nullptr, out, n_out, out_legs);
-    return tncb::execute(ctx, plan->S, nullptr, out, n_out, out_legs, (const double2*)((char*)plan->ws + plan->leaf_off));
+    return tncb::execute(ctx, plan->S, nullptr, out, n_out, out_legs, (char*)plan->ws + plan->leaf_off);
   }
   if (!plan->resident || plan->ctx != ctx) return tncb::fail(TNCB_ERR_INVALID, "tncb_plan_stage has not been called on this context");
-  return tncb::execute(ctx, plan->S, nullptr, out, n_out, out_legs, (const double2*)plan->resident);
+  return tncb::execute(ctx, plan->S, nullptr, out, n_out, out_legs, plan->resident);
 }
 
 // Sliced execution (the reference's declared future work, book/src/future_work.md:9-11) without host work per slice:
@@ -726,8 +759,8 @@ int tncb_plan_stage_slices(tncb_ctx* ctx, tncb_plan* plan, size_t n_slices, cons
   TNCB_CUDA(cudaSetDevice(ctx->device));
   int rc;
   if ((rc = tncb::plan_device_state(ctx, plan))) return rc;
-  const size_t block = std::max<size_t>(S.leaf_block_elems, 1);
-  std::vector<std::complex<double>> host(block * n_slices);
+  const size_t block = std::max<size_t>(S.leaf_block_elems, 1) * S.esz();   // bytes per slice
+  std::vector<char> host(block * n_slices);
   for (size_t q = 0; q < n_slices; q++) {
     if (!slice_tns[q]) return tncb::fail(TNCB_ERR_INVALID, "slice network is null");
     std::vector<const tncb_tn*> leaves;
@@ -737,7 +770,7 @@ int tncb_plan_stage_slices(tncb_ctx* ctx, tncb_plan* plan, size_t n_slices, cons
   }
   TNCB_CUDA(cudaStreamSynchronize(ctx->stream));
   if (plan->slices_dev) { ctx->arena.free(plan->slices_dev, plan->slices_bytes); plan->slices_dev = nullptr; }
-  plan->slices_bytes = host.size() * sizeof(double2);
+  plan->slices_bytes = host.size();
   if ((rc = ctx->arena.alloc(plan->slices_bytes, &plan->slices_dev))) return rc;
   TNCB_CUDA(cudaMemcpyAsync(plan->slices_dev, host.data(), plan->slices_bytes, cudaMemcpyHostToDevice, ctx->stream));
   TNCB_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -753,9 +786,10 @@ int tncb_plan_run_slices(tncb_ctx* ctx, tncb_plan* plan, size_t first, size_t st
   TNCB_CUDA(cudaSetDevice(ctx->device));
   const tncb::SlotMeta& rm = S.slots[S.result_slot];
   tncb_tensor* sum = nullptr;
-  int rc = tncb::tensor_new(ctx, (int)rm.dims.size(), rm.dims.data(), &sum);
+  int rc = tncb::tensor_new(ctx, (int)rm.dims.size(), rm.dims.data(), &sum, S.dtype);
   if (rc) return rc;
-  const size_t block_bytes = std::max<size_t>(S.leaf_block_elems, 1) * sizeof(double2);
+  const size_t esz = S.esz();
+  const size_t block_bytes = std::max<size_t>(S.leaf_block_elems, 1) * esz;
   char* ws = (char*)plan->ws;
   bool any = false;
   for (size_t q = first; q < plan->n_slices; q += stride) {
@@ -764,12 +798,12 @@ int tncb_plan_run_slices(tncb_ctx* ctx, tncb_plan* plan, size_t first, size_t st
     tncb_tensor* part = nullptr;
     if ((rc = tncb::execute_static(ctx, plan, nullptr, &part, nullptr, nullptr))) { tncb_tensor_free(ctx, sum); return rc; }
     if (!any) {
-      TNCB_CUDA(cudaMemcpyAsync(sum->ptr, part->ptr, rm.elems * sizeof(double2), cudaMemcpyDeviceToDevice, ctx->stream));
+      TNCB_CUDA(cudaMemcpyAsync(sum->ptr, part->ptr, rm.elems * esz, cudaMemcpyDeviceToDevice, ctx->stream));
       any = true;
-    } else if ((rc = tncb::launch_add(ctx, sum->ptr, part->ptr, rm.elems))) { tncb_tensor_free(ctx, part); tncb_tensor_free(ctx, sum); return rc; }
+    } else if ((rc = tncb::launch_add(ctx, sum->ptr, part->ptr, rm.elems, S.dtype))) { tncb_tensor_free(ctx, part); tncb_tensor_free(ctx, sum); return rc; }
     tncb_tensor_free(ctx, part);
   }
-  if (!any) TNCB_CUDA(cudaMemsetAsync(sum->ptr, 0, std::max<size_t>(rm.elems, 1) * sizeof(double2), ctx->stream));   // more ranks than slices
+  if (!any) TNCB_CUDA(cudaMemsetAsync(sum->ptr, 0, std::max<size_t>(rm.elems, 1) * esz, ctx->stream));   // more ranks than slices
   if (out) *out = sum; else tncb_tensor_free(ctx, sum);
   if (n_out) *n_out = (int)rm.legs.size();
   if (out_legs) for (size_t i = 0; i < rm.legs.size(); i++) out_legs[i] = rm.legs[i];
@@ -798,13 +832,14 @@ int tncb_plan_info(const tncb_plan* plan, uint64_t* n_pairs, double* flops, doub
   if (!plan) return tncb::fail(TNCB_ERR_INVALID, "plan is null");
   const tncb::Schedule& S = plan->S;
   if (n_pairs) *n_pairs = S.steps.size();
+  const size_t esz = S.esz();
   if (flops) *flops = S.flops;
-  if (bytes) *bytes = S.bytes;
+  if (bytes) *bytes = S.bytes * (double)esz / 16.0;
   if (peak_bytes) { // replay the liveness: leaves + live intermediates
-    size_t live = S.leaf_block_elems * 16, peak = live;
+    size_t live = S.leaf_block_elems * esz, peak = live;
     std::vector<size_t> sz(S.slots.size(), 0);
     for (const tncb::Step& st : S.steps) {
-      sz[st.out] = std::max<size_t>(S.slots[st.out].elems * 16, 256);
+      sz[st.out] = std::max<size_t>(S.slots[st.out].elems * esz, 256);
       live += sz[st.out]; peak = std::max(peak, live);
       live -= sz[st.a] + sz[st.b]; sz[st.a] = sz[st.b] = 0;
     }

@@ -109,12 +109,13 @@ void gemm_timer_end(tncb_ctx* ctx, double ops) {
   }
 }
 
-int tensor_new(tncb_ctx* ctx, int rank, const uint64_t* dims, tncb_tensor** out) {
+int tensor_new(tncb_ctx* ctx, int rank, const uint64_t* dims, tncb_tensor** out, int dtype) {
   if (rank < 0 || rank > kMaxLegs) return fail(TNCB_ERR_INVALID, "tensor rank out of range");
+  if (!dtype_size(dtype)) return fail(TNCB_ERR_INVALID, "dtype must be TNCB_C128 or TNCB_C64");
   tncb_tensor* t = new tncb_tensor();
-  t->rank = rank; t->elems = 1;
+  t->rank = rank; t->elems = 1; t->dtype = dtype;
   for (int i = 0; i < rank; i++) { t->dims[i] = dims[i]; t->elems *= dims[i]; }
-  t->bytes = std::max<size_t>(t->elems * sizeof(double2), 16);
+  t->bytes = std::max<size_t>(t->elems * dtype_size(dtype), 16);
   void* p = nullptr;
   int rc = ctx->arena.alloc(t->bytes, &p);
   if (rc) { delete t; return rc; }
@@ -402,27 +403,39 @@ int tncb_ctx_last_gemm_ms(tncb_ctx* ctx, float* ms) {
   return TNCB_OK;
 }
 
-int tncb_tensor_alloc(tncb_ctx* ctx, int rank, const uint64_t* dims, tncb_tensor** out) {
+int tncb_tensor_alloc_dt(tncb_ctx* ctx, int rank, const uint64_t* dims, int dtype, tncb_tensor** out) {
   if (!ctx || !out || (rank > 0 && !dims)) return fail(TNCB_ERR_INVALID, "null argument");
+  if (!dtype_size(dtype)) return fail(TNCB_ERR_INVALID, "dtype must be TNCB_C128 or TNCB_C64");
   TNCB_CUDA(cudaSetDevice(ctx->device));
-  return tensor_new(ctx, rank, dims, out);
+  return tensor_new(ctx, rank, dims, out, dtype);
 }
 
-int tncb_tensor_upload(tncb_ctx* ctx, int rank, const uint64_t* dims, const double* host, tncb_tensor** out) {
+int tncb_tensor_alloc(tncb_ctx* ctx, int rank, const uint64_t* dims, tncb_tensor** out) {
+  return tncb_tensor_alloc_dt(ctx, rank, dims, TNCB_C128, out);
+}
+
+int tncb_tensor_upload_dt(tncb_ctx* ctx, int rank, const uint64_t* dims, int dtype, const void* host, tncb_tensor** out) {
   if (!host) return fail(TNCB_ERR_INVALID, "host buffer is null");
-  int rc = tncb_tensor_alloc(ctx, rank, dims, out);
+  int rc = tncb_tensor_alloc_dt(ctx, rank, dims, dtype, out);
   if (rc) return rc;
   tncb_tensor* t = *out;
   // pageable or pinned host memory both work; the copy is ordered on the ctx stream
-  TNCB_CUDA(cudaMemcpyAsync(t->ptr, host, t->elems * sizeof(double2), cudaMemcpyHostToDevice, ctx->stream));
+  TNCB_CUDA(cudaMemcpyAsync(t->ptr, host, t->elems * dtype_size(dtype), cudaMemcpyHostToDevice, ctx->stream));
   TNCB_CUDA(cudaStreamSynchronize(ctx->stream));
   return TNCB_OK;
 }
 
+int tncb_tensor_upload(tncb_ctx* ctx, int rank, const uint64_t* dims, const double* host, tncb_tensor** out) {
+  return tncb_tensor_upload_dt(ctx, rank, dims, TNCB_C128, host, out);
+}
+
+int tncb_tensor_dtype(const tncb_tensor* t) { return t ? t->dtype : TNCB_ERR_INVALID; }
+
+// raw copies in the tensor's own dtype
 int tncb_tensor_download(tncb_ctx* ctx, const tncb_tensor* t, double* host) {
   if (!ctx || !t || !host) return fail(TNCB_ERR_INVALID, "null argument");
   TNCB_CUDA(cudaSetDevice(ctx->device));
-  TNCB_CUDA(cudaMemcpyAsync(host, t->ptr, t->elems * sizeof(double2), cudaMemcpyDeviceToHost, ctx->stream));
+  TNCB_CUDA(cudaMemcpyAsync(host, t->ptr, t->elems * dtype_size(t->dtype), cudaMemcpyDeviceToHost, ctx->stream));
   TNCB_CUDA(cudaStreamSynchronize(ctx->stream));
   return TNCB_OK;
 }
@@ -430,14 +443,14 @@ int tncb_tensor_download(tncb_ctx* ctx, const tncb_tensor* t, double* host) {
 int tncb_tensor_write(tncb_ctx* ctx, tncb_tensor* t, const double* host) {
   if (!ctx || !t || !host) return fail(TNCB_ERR_INVALID, "null argument");
   TNCB_CUDA(cudaSetDevice(ctx->device));
-  TNCB_CUDA(cudaMemcpyAsync(t->ptr, host, t->elems * sizeof(double2), cudaMemcpyHostToDevice, ctx->stream));
+  TNCB_CUDA(cudaMemcpyAsync(t->ptr, host, t->elems * dtype_size(t->dtype), cudaMemcpyHostToDevice, ctx->stream));
   return TNCB_OK;
 }
 
 int tncb_tensor_read(tncb_ctx* ctx, const tncb_tensor* t, double* host) {
   if (!ctx || !t || !host) return fail(TNCB_ERR_INVALID, "null argument");
   TNCB_CUDA(cudaSetDevice(ctx->device));
-  TNCB_CUDA(cudaMemcpyAsync(host, t->ptr, t->elems * sizeof(double2), cudaMemcpyDeviceToHost, ctx->stream));
+  TNCB_CUDA(cudaMemcpyAsync(host, t->ptr, t->elems * dtype_size(t->dtype), cudaMemcpyDeviceToHost, ctx->stream));
   return TNCB_OK;
 }
 
@@ -466,16 +479,23 @@ static int check_tensor_legs(const tncb_tensor* t, int n, const char* who) {
   return TNCB_OK;
 }
 
+// no implicit promotion: every tensor of one call has the same dtype
+static int check_same_dtype(const tncb_tensor* a, const tncb_tensor* b) {
+  if (a->dtype != b->dtype) return fail(TNCB_ERR_INVALID, "operands have different dtypes (complex64 vs complex128)");
+  return TNCB_OK;
+}
+
 int tncb_contract_pair_into(tncb_ctx* ctx, int n_a, const uint64_t* a_legs, const tncb_tensor* a,
                             int n_b, const uint64_t* b_legs, const tncb_tensor* b, tncb_tensor* out) {
   if (!ctx || !out) return fail(TNCB_ERR_INVALID, "null argument");
   int rc;
   if ((rc = check_tensor_legs(a, n_a, "a")) || (rc = check_tensor_legs(b, n_b, "b"))) return rc;
+  if ((rc = check_same_dtype(a, b)) || (rc = check_same_dtype(a, out))) return rc;
   TNCB_CUDA(cudaSetDevice(ctx->device));
   PairPlan P;
   if ((rc = plan_pair(n_a, a_legs, a->dims, n_b, b_legs, b->dims, P))) return rc;
   if ((uint64_t)(P.M * P.N) != out->elems) return fail(TNCB_ERR_SHAPE, "output tensor has the wrong number of elements");
-  return launch_pair(ctx, P, a->ptr, b->ptr, out->ptr);
+  return launch_pair(ctx, P, a->ptr, b->ptr, out->ptr, a->dtype);
 }
 
 int tncb_contract_pair_keep(tncb_ctx* ctx, int n_a, const uint64_t* a_legs, const tncb_tensor* a,
@@ -483,12 +503,13 @@ int tncb_contract_pair_keep(tncb_ctx* ctx, int n_a, const uint64_t* a_legs, cons
   if (!ctx || !out) return fail(TNCB_ERR_INVALID, "null argument");
   int rc;
   if ((rc = check_tensor_legs(a, n_a, "a")) || (rc = check_tensor_legs(b, n_b, "b"))) return rc;
+  if ((rc = check_same_dtype(a, b))) return rc;
   TNCB_CUDA(cudaSetDevice(ctx->device));
   PairPlan P;
   if ((rc = plan_pair(n_a, a_legs, a->dims, n_b, b_legs, b->dims, P))) return rc;
   tncb_tensor* c = nullptr;
-  if ((rc = tensor_new(ctx, (int)P.out_dims.size(), P.out_dims.data(), &c))) return rc;
-  if ((rc = launch_pair(ctx, P, a->ptr, b->ptr, c->ptr))) { tncb_tensor_free(ctx, c); return rc; }
+  if ((rc = tensor_new(ctx, (int)P.out_dims.size(), P.out_dims.data(), &c, a->dtype))) return rc;
+  if ((rc = launch_pair(ctx, P, a->ptr, b->ptr, c->ptr, a->dtype))) { tncb_tensor_free(ctx, c); return rc; }
   *out = c;
   return TNCB_OK;
 }
@@ -500,6 +521,7 @@ int tncb_contract_pair(tncb_ctx* ctx, int n_out, const uint64_t* out_legs,
   int rc;
   if ((rc = check_tensor_legs(a, n_a, "a")) || (rc = check_tensor_legs(b, n_b, "b"))) return rc;
   if (a == b) return fail(TNCB_ERR_INVALID, "a and b are the same tensor");
+  if ((rc = check_same_dtype(a, b))) return rc;
   if (out_legs) {
     PairPlan P;
     if ((rc = plan_pair(n_a, a_legs, a->dims, n_b, b_legs, b->dims, P))) return rc;
@@ -525,9 +547,9 @@ int tncb_permute(tncb_ctx* ctx, tncb_tensor* t, const int* perm, tncb_tensor** o
     seen[perm[i]] = true; odims[i] = t->dims[perm[i]];
   }
   tncb_tensor* o = nullptr;
-  int rc = tensor_new(ctx, t->rank, odims, &o);
+  int rc = tensor_new(ctx, t->rank, odims, &o, t->dtype);
   if (rc) return rc;
-  if ((rc = launch_permute(ctx, t->ptr, o->ptr, t->rank, t->dims, perm))) { tncb_tensor_free(ctx, o); return rc; }
+  if ((rc = launch_permute(ctx, t->ptr, o->ptr, t->rank, t->dims, perm, t->dtype))) { tncb_tensor_free(ctx, o); return rc; }
   tncb_tensor_free(ctx, t);
   *out = o;
   return TNCB_OK;
@@ -535,15 +557,17 @@ int tncb_permute(tncb_ctx* ctx, tncb_tensor* t, const int* perm, tncb_tensor** o
 
 int tncb_tensor_add(tncb_ctx* ctx, tncb_tensor* dst, const tncb_tensor* src) {
   if (!ctx || !dst || !src) return fail(TNCB_ERR_INVALID, "null argument");
+  int rc;
+  if ((rc = check_same_dtype(dst, src))) return rc;
   if (dst->elems != src->elems) return fail(TNCB_ERR_SHAPE, "tensor_add: element counts differ");
   TNCB_CUDA(cudaSetDevice(ctx->device));
-  return launch_add(ctx, dst->ptr, src->ptr, dst->elems);
+  return launch_add(ctx, dst->ptr, src->ptr, dst->elems, dst->dtype);
 }
 
 int tncb_conjugate(tncb_ctx* ctx, tncb_tensor* t) {
   if (!ctx || !t) return fail(TNCB_ERR_INVALID, "null argument");
   TNCB_CUDA(cudaSetDevice(ctx->device));
-  return launch_conj(ctx, t->ptr, t->elems);
+  return launch_conj(ctx, t->ptr, t->elems, t->dtype);
 }
 
 } // extern "C"

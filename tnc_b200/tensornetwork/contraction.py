@@ -12,7 +12,7 @@ from typing import List, Optional
 
 import numpy as np
 
-from .. import Context, DeviceTensor, default_context
+from .. import Context, DeviceTensor, default_context, dtype_code
 from .._lib import TncbError, TncbPath, TncbTn, check, u64_array
 from ..contractionpath import ContractionPath
 from .tensor import Tensor
@@ -145,9 +145,13 @@ class _Marshal:
         return out
 
 
-def contract_tensor_network(tn: Tensor, contract_path: ContractionPath, ctx: Optional[Context] = None) -> Tensor:
+def contract_tensor_network(tn: Tensor, contract_path: ContractionPath, ctx: Optional[Context] = None,
+                            dtype=np.complex128) -> Tensor:
     """Fully contracts `tn` with the replace-left `contract_path`; returns the resulting
-    leaf `Tensor` whose data stays on the device (`.to_numpy()` downloads it)."""
+    leaf `Tensor` whose data stays on the device (`.to_numpy()` downloads it).
+    dtype=np.complex64 runs every kernel in complex64 (f64 accumulation, one rounding per result; host payloads are
+    narrowed while they are staged, device leaves must already be complex64); the result is complex64 then."""
+    code = dtype_code(dtype)
     ctx = ctx or default_context()
     m = _Marshal()
     c_tn = m.tn(tn)
@@ -155,7 +159,7 @@ def contract_tensor_network(tn: Tensor, contract_path: ContractionPath, ctx: Opt
     out = C.c_void_p()
     n_out = C.c_int()
     legs = u64_array([0] * 64)
-    rc = ctx._l.tncb_contract_tensor_network(ctx.handle, C.byref(c_tn), C.byref(c_path), C.byref(out), C.byref(n_out), legs)
+    rc = ctx._l.tncb_contract_tensor_network_dt(ctx.handle, C.byref(c_tn), C.byref(c_path), code, C.byref(out), C.byref(n_out), legs)
     check(rc)
     for d in m.device_inputs:  # consumed by the call
         d.release()
@@ -168,14 +172,18 @@ def contract_tensor_network(tn: Tensor, contract_path: ContractionPath, ctx: Opt
 
 
 class NetworkPlan:
-    """Compile once / execute many (tncb_plan_*): same structure, new payloads."""
+    """Compile once / execute many (tncb_plan_*): same structure, new payloads.  `dtype` (complex128 or complex64) is the
+    element type of every run of the plan."""
 
-    def __init__(self, tn: Tensor, contract_path: ContractionPath, ctx: Optional[Context] = None):
+    def __init__(self, tn: Tensor, contract_path: ContractionPath, ctx: Optional[Context] = None, dtype=np.complex128):
+        self.handle = None
+        code = dtype_code(dtype)
+        self.dtype = np.dtype(dtype)
         self.ctx = ctx or default_context()
         m = _Marshal()
         c_tn, c_path = m.tn(tn), m.path(contract_path)
         h = C.c_void_p()
-        check(self.ctx._l.tncb_plan_create(self.ctx.handle, C.byref(c_tn), C.byref(c_path), C.byref(h)))
+        check(self.ctx._l.tncb_plan_create_dt(self.ctx.handle, C.byref(c_tn), C.byref(c_path), code, C.byref(h)))
         self.handle = h
 
     def info(self) -> dict:
